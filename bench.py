@@ -3,6 +3,7 @@
 Benchmark of the bundle-adjustment hot path (see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2|1m|small|cfg3|cfg3a|cfg4s]
+                    [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one trust-region (Levenberg-Marquardt) iteration of the
 workload the metric is quoted on ("LM iters/s and Jacobian obs/s at 1M obs"): BASELINE config 2 at twice its
@@ -19,6 +20,11 @@ and the per-iteration exchange is the SUM all-reduce of the partial camera syste
             measured HBM copy bandwidth of MEASURED_PEAKS.json
   cpu_baseline = the reference's path (oracle port: numpy residual + scipy TRF/2-point/LSMR) on this box's CPU
 `--impl reference` times that CPU path alone, in the same unit, on the same workload.
+`--dump-outputs DIR` writes what the last timed solve returned (camera and point variables, cost) as .npy files; the
+inputs are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
+Beyond 25 steps the timed iterations run as several solves of at most 25 iterations that each restart from the same
+start (with W untimed iterations first), and the dump is the result of the last one: compare dumps taken with the same
+--steps and --warmup.
 """
 import argparse
 import json
@@ -61,6 +67,7 @@ WORKLOADS = {
 RPC_WORKLOAD = "rpc"         # BASELINE config 5: RPC refit + batched RPC projection / localisation / triangulation, 300 cameras
 LS = {"loss": "soft_l1", "f_scale": 1.0}
 L2_FLUSH_BYTES = 256 << 20      # > 126 MB L2
+DUMP_LIMIT_BYTES = 64 * 10 ** 6  # --dump-outputs writes at most this much
 
 
 def load_peaks():
@@ -183,6 +190,18 @@ def algorithmic_bytes(K, N, M, c, engine):
     }
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each array of `arrays` (name -> array) as out_dir/<name>.npy in float64.  The largest output of any workload
+    (1e6 tracks on one GPU: 24 MB) fits DUMP_LIMIT_BYTES whole, so nothing is sampled."""
+    arrays = {name: np.ascontiguousarray(a, dtype=np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes + 1024 for a in arrays.values())       # + room for each .npy header
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes of outputs exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def fp64_peak():
     """Measured FP64 FMA peak of this pool's B200 (tools/fp64_peak.cu, committed result profiles/r02_fp64_peak.json)."""
     path = os.path.join(ROOT, "profiles", "r02_fp64_peak.json")
@@ -278,9 +297,10 @@ def run_reference_arm(args):
 # ---------------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------------
-def measure_workload(workload, K, W, world, rank, local_rank, with_e2e=True, with_clocks=True):
+def measure_workload(workload, K, W, world, rank, local_rank, with_e2e=True, with_clocks=True, keep_outputs=False):
     """Device-timed iterations (+ phases), the fused Jacobian/assembly pass alone and the end-to-end call for one workload.
-    Returns a dict of raw measurements on every rank (max over ranks already taken)."""
+    Returns a dict of raw measurements on every rank (max over ranks already taken); with keep_outputs, also what the last
+    timed solve computed ("outputs")."""
     import torch
     import torch.distributed as dist
     from sat_bundleadjust_b200 import ba_core
@@ -331,6 +351,7 @@ def measure_workload(workload, K, W, world, rank, local_rank, with_e2e=True, wit
                                      no_phase_timing=no_phase_timing, **LS)
             assert part["timed_iterations"] == k, part
             per_it.append(part["iter_ms"] / k)
+            last_cost = part["cost"]
             if acc is None:
                 acc = part
             else:
@@ -341,12 +362,16 @@ def measure_workload(workload, K, W, world, rank, local_rank, with_e2e=True, wit
                     acc["phase_ms"][ph] += part["phase_ms"][ph]
             left -= k
         acc["segment_ms_per_iteration"] = per_it
+        acc["last_cost"] = last_cost
         return acc
 
     # the headline: whole iterations only (one CUDA-event pair per iteration); then the same K iterations again with the
     # per-phase events on (more event records per iteration, which themselves cost ~1 us each on the stream)
     info = timed_run(1)
     barrier()
+    # what the headline's last solve returned to its caller: the variables in the device layout (cameras, then this rank's
+    # tracks) and the cost
+    x_last = out_dev.cpu().numpy() if keep_outputs else None
     info_ph = timed_run(0)
     barrier()
     keys = list(info_ph["phase_ms"].keys())
@@ -374,6 +399,9 @@ def measure_workload(workload, K, W, world, rank, local_rank, with_e2e=True, wit
            "jac_ms": float(jac.item()), "gpu_launches": int(info["gpu_launches"]), "n_obs_local": prob.n_obs,
            "n_pts_local": prob.n_pts, "n_vars_local": prob.n_vars, "segments": info["segment_ms_per_iteration"],
            "clocks": sampler.stop() if sampler else None}
+    if keep_outputs:
+        out["outputs"] = {"cameras": x_last[:ncv].reshape(p.n_cam, p.n_params), "points": x_last[ncv:].reshape(-1, 3),
+                          "cost": np.array([info["last_cost"]])}
     if world > 1:
         dist.barrier()      # peers may still be reading this rank's exchange buffer
     prob.close()
@@ -430,7 +458,9 @@ def run_b200_arm(args):
             os.environ["NCCL_DEBUG"] = "WARN"      # keep NCCL's version banner off stdout: one JSON line only
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     W, K = args.warmup, args.steps
-    m = measure_workload(args.workload, K, W, world, rank, local_rank)
+    m = measure_workload(args.workload, K, W, world, rank, local_rank, keep_outputs=args.dump_outputs is not None)
+    if rank == 0 and args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, m["outputs"])
     second = None
     if world == 1 and not args.no_secondary and args.workload != "cfg2":
         second = measure_workload("cfg2", K, W, world, rank, local_rank, with_e2e=True, with_clocks=False)
@@ -527,7 +557,7 @@ def run_rpc_workload(args):
         return 0
     G = np.load(os.path.join(ROOT, "tests", "golden", "rpc_golden.npz"))
     F = np.load(os.path.join(ROOT, "tests", "golden", "rpcfit_golden.npz"))
-    n_cam, reps = 300, max(1, args.steps // 4)
+    n_cam, reps = 300, args.steps                           # timed passes of each batched operation (after one untimed pass)
     rng = np.random.default_rng(0)
     base = [G["rpc_a"], G["rpc_b"]]
     tables = np.stack([base[j % 2].copy() for j in range(2 * n_cam)])
@@ -589,6 +619,9 @@ def run_rpc_workload(args):
     assert np.abs(o[:n] - last.projection(lon, lat, alt)[0]).max() < 1e-6
     ms_loc, o = thr(1, f64(col_a), f64(row_a), f64(alt), None, 1.0, 2)
     ms_tri, o = thr(2, f64(col_a), f64(row_a), f64(col_b), f64(row_b), 0.1, 3)
+    if args.dump_outputs is not None:
+        # the headline's last pass: lon, lat, alt of every match of the last camera pair
+        dump_outputs(args.dump_outputs, {"triangulation_lonlatalt": o.reshape(n, 3)})
     # refit: 300 cameras x 1000 samples through the public batched call (host buffers in and out)
     tg = np.stack([F["case%d/target" % (k % int(F["n_cases"]))] for k in range(n_cam)])
     lc = np.stack([F["case%d/input_locs" % (k % int(F["n_cases"]))] for k in range(n_cam)])
@@ -669,7 +702,14 @@ def main():
     ap.add_argument("--workload", default="1m", choices=sorted(WORKLOADS) + [RPC_WORKLOAD])
     ap.add_argument("--no-secondary", action="store_true", help="skip the config-2 line reported under \"secondary\" (N = 1)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed solve returned as DIR/<name>.npy (float64, "
+                    "at most 64 MB in all; at N > 1, rank 0's cameras and tracks).  Beyond 25 steps that solve restarts from "
+                    "the initial point, so compare dumps taken with the same --steps and --warmup.  bench_outputs/ is git-ignored")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 0)
     if args.workload == RPC_WORKLOAD:
         rc = run_rpc_workload(args)

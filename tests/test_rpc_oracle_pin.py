@@ -18,7 +18,8 @@ def test_projection_bit_exact():
         col, row = rpc.projection(lla[:, 0], lla[:, 1], lla[:, 2])
         assert np.array_equal(np.stack((col, row), axis=1), R[key])
     port = rpc_ctypes.load_port()
-    assert np.array_equal(rpc_ctypes.port_project(port, RA, lla), R["ref_proj_a"])
+    for rpc, key in ((RA, "ref_proj_a"), (RB, "ref_proj_b")):       # the C port against the compiled reference's output
+        assert np.array_equal(rpc_ctypes.port_project(port, rpc, lla), R[key]), key
 
 
 def test_localization_bit_exact():
