@@ -156,6 +156,25 @@ int sba_normal_blocks(sba_problem *p, const double *x, int32_t loss, double f_sc
  * counterpart: the reference never forms S).  Host buffers; S is (n_cam n_params)^2, column-major. */
 int sba_reduced_system(sba_problem *p, const double *x, int32_t loss, double f_scale, double reg, double *S, double *rhs);
 
+/* Posterior covariance at x (host pointers, caller's layouts).  sigma2 > 0: used as given; else estimated and
+ * returned in *sigma2_out.  cov_cam (M*n_params)^2 column-major, cov_pts (N,6); either may be NULL.
+ * SBA_E_INVALID: world_size > 1, PCG problems (no dense S), n_common > 0, dof <= 0.
+ * SBA_E_NUMERIC: rank-deficient S (gauge not fixed) or a free point with a singular block.
+ * J is the Jacobian of the weighted residuals at x over the free variables, rescaled for the robust loss like the solver does
+ * (scipy's scale_for_robust_loss_function); H = J^T J = [[U, W], [W^T, V]], S = U - W V^-1 W^T.  cov_cam = sigma2 S^-1 (rows
+ * and columns of frozen cameras 0); cov_pts[t] = sigma2 (V_t^-1 + V_t^-1 W_t^T S^-1 W_t V_t^-1) as xx xy xz yy yz zz (frozen
+ * points 0).  Estimated sigma2 = 2 cost(x) / (2K - n_free) (scipy curve_fit's convention).  S is rejected as rank deficient
+ * when a pivot of its Cholesky factor has L_kk^2 <= 1e-12 U_kk; *min_pivot_ratio_out (may be NULL) receives the smallest
+ * L_kk^2 / U_kk over the free camera slots.  The pivot test catches round-off pivots, it does not certify full rank: in
+ * ill-conditioned geometry a single free direction (e.g. the scale left by one frozen perspective camera) can pass it, so
+ * fix the gauge with at least two frozen cameras or with frozen points.  The handle stays usable for solves, also after an
+ * error return. */
+int sba_covariance(sba_problem *p, const double *x, int32_t loss, double f_scale, double sigma2,
+                   double *cov_cam, double *cov_pts, double *sigma2_out, double *min_pivot_ratio_out);
+/* Device time (CUDA events) of the phases of the last sba_covariance call on this handle: reduced system (assembly, Schur
+ * pass, cost), factorisation + pivot test, inverse, point pass. */
+int sba_covariance_phase_ms(const sba_problem *p, double ms_out[4]);
+
 /* Replaces scipy.optimize.least_squares(fun, x0, jac_sparsity=A, x_scale='jac', method='trf', ...)
  * as called by ba_core.run_ba_optimization (ba_core.py:284-297).
  * x0 (n) in, x (n) out, r (2K) = un-scaled residuals at the solution (res.fun), may be NULL. */

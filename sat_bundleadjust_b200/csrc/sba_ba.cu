@@ -25,6 +25,7 @@
 #include <vector>
 
 #include "sba_comm.cuh"
+#include "sba_cov.cuh"
 #include "sba_index.h"
 #include "sba_kernels.cuh"
 #include "sba_pattern.cuh"
@@ -817,6 +818,7 @@ extern "C" int sba_problem_destroy(sba_problem* p)
     if (p->ev_join) cudaEventDestroy(p->ev_join);
     if (p->stream2) cudaStreamDestroy(p->stream2);
     for (cudaEvent_t e : p->ev_pool) cudaEventDestroy(e);
+    for (cudaEvent_t e : p->cov_ev) if (e) cudaEventDestroy(e);
     if (p->flush_buf) cudaFree(p->flush_buf);
     delete p;
     return SBA_OK;
@@ -1259,15 +1261,14 @@ extern "C" int sba_normal_blocks(sba_problem* p, const double* x, int32_t loss, 
 // The reduced camera system of the damped normal equations at x, as the solver forms it (scaling D from this one
 // evaluation): S = U + reg D_c^2 - W (V + reg D_p^2)^-1 W^T and rhs = -(g_c - W (V + reg D_p^2)^-1 g_p), COMMON_K folded.
 // Exposed for the parity tests of the Schur complement; host buffers, S is (M n_params)^2 column-major.
-extern "C" int sba_reduced_system(sba_problem* p, const double* x, int32_t loss, double f_scale, double reg, double* S,
-                                  double* rhs)
+// Device part: x (host) is uploaded (then `uploaded`, if given, is recorded); afterwards p->x / p->camrec hold x, p->camsys its
+// U blocks, p->S the system, and the cost at x is in scal[SC_COST_NEW] (pattern engine) or scal[SC_COST] (generic engine).
+static int form_reduced_system(sba_problem* p, const double* x, int32_t loss, double f_scale, double reg,
+                               cudaEvent_t uploaded = nullptr)
 {
-    if (!p || !x || !S || !rhs || !(reg >= 0.0)) { set_error("bad argument"); return SBA_E_INVALID; }
-    if (p->world > 1) { set_error("sba_reduced_system: single-rank problems only"); return SBA_E_INVALID; }
-    SBA_CUDA(cudaSetDevice(p->device));
-    const size_t ns = (size_t)p->M * p->nc;
     if (p->engine == 1) {
         SBA_CUDA(cudaMemcpyAsync(p->io_x, x, (size_t)p->n * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+        if (uploaded) SBA_CUDA(cudaEventRecord(uploaded, p->stream));
         SBA_TRY(vars_in(p, p->io_x, p->x));
         SBA_TRY(pt_reset_state(p));
         SBA_TRY(pt_run_assemble(p, 1, 1, loss, f_scale));
@@ -1279,6 +1280,7 @@ extern "C" int sba_reduced_system(sba_problem* p, const double* x, int32_t loss,
     } else {
         SBA_CUDA(cudaMemsetAsync(p->scal, 0, SC_COUNT * sizeof(double), p->stream));
         SBA_CUDA(cudaMemcpyAsync(p->x, x, (size_t)p->n * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+        if (uploaded) SBA_CUDA(cudaEventRecord(uploaded, p->stream));
         SBA_TRY(run_prepare(p, p->x, p->camrec));
         SBA_TRY(run_assemble(p, p->x, p->camrec, loss, f_scale));
         SBA_TRY(run_scale_dots(p, 1));
@@ -1288,9 +1290,169 @@ extern "C" int sba_reduced_system(sba_problem* p, const double* x, int32_t loss,
         tm.p = p;
         SBA_TRY(run_gauss_newton_step(p, loss, f_scale, tm, true));
     }
+    return SBA_OK;
+}
+
+extern "C" int sba_reduced_system(sba_problem* p, const double* x, int32_t loss, double f_scale, double reg, double* S,
+                                  double* rhs)
+{
+    if (!p || !x || !S || !rhs || !(reg >= 0.0)) { set_error("bad argument"); return SBA_E_INVALID; }
+    if (p->world > 1) { set_error("sba_reduced_system: single-rank problems only"); return SBA_E_INVALID; }
+    SBA_CUDA(cudaSetDevice(p->device));
+    const size_t ns = (size_t)p->M * p->nc;
+    SBA_TRY(form_reduced_system(p, x, loss, f_scale, reg));
     SBA_CUDA(cudaMemcpyAsync(S, p->S, ns * ns * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     SBA_CUDA(cudaMemcpyAsync(rhs, p->S + ns * ns, ns * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
     SBA_CUDA(cudaStreamSynchronize(p->stream));
+    return SBA_OK;
+}
+
+// Posterior covariance at x (sba_cov.cuh has the definitions): the undamped reduced camera system through the solver's own
+// Schur path, its Cholesky factor with the pivot test, S^-1, then one pass over the tracks.
+constexpr double COV_PIVOT_THRESHOLD = 1e-12;
+constexpr size_t COV_SMEM_MAX = 100 * 1024;     // s2 S^-1 goes to shared memory up to this size (ns <= 113)
+
+// Warp tiles of the point pass in the internal track order (runs of whole tracks of <= 32 observations, a longer track a tile
+// of its own): the generic engine has them; the pattern engine's are built once, on the first call, from its track offsets.
+static int cov_tiles(sba_problem* p, const int** tiles, int* n_tiles)
+{
+    if (p->engine == 0) { *tiles = p->tile_obs; *n_tiles = p->n_tiles; return SBA_OK; }
+    if (!p->cov_tile_obs) {
+        std::vector<int> tp((size_t)p->N + 1), to(1, 0);
+        SBA_CUDA(cudaMemcpyAsync(tp.data(), p->track_ptr, tp.size() * sizeof(int), cudaMemcpyDeviceToHost, p->stream));
+        SBA_CUDA(cudaStreamSynchronize(p->stream));
+        int cur = 0;
+        for (int i = 0; i < p->N; ++i) {
+            const int L = tp[i + 1] - tp[i];
+            if (L == 0) continue;
+            if (cur > 0 && cur + L > 32) { to.push_back(tp[i]); cur = 0; }
+            cur += L;
+            if (cur >= 32) { to.push_back(tp[i + 1]); cur = 0; }
+        }
+        if (cur > 0) to.push_back(tp[p->N]);
+        SBA_TRY(dev_upload(p, &p->cov_tile_obs, to, p->stream));
+        SBA_CUDA(cudaStreamSynchronize(p->stream));
+        p->cov_n_tiles = (int)to.size() - 1;
+    }
+    *tiles = p->cov_tile_obs; *n_tiles = p->cov_n_tiles;
+    return SBA_OK;
+}
+
+extern "C" int sba_covariance(sba_problem* p, const double* x, int32_t loss, double f_scale, double sigma2, double* cov_cam,
+                              double* cov_pts, double* sigma2_out, double* min_pivot_ratio_out)
+{
+    if (!p || !x) { set_error("null argument"); return SBA_E_INVALID; }
+    if (p->world > 1) { set_error("sba_covariance: single-rank problems only"); return SBA_E_INVALID; }
+    if (p->use_pcg) { set_error("sba_covariance: the PCG path forms no dense reduced camera system"); return SBA_E_INVALID; }
+    if (p->n_common) { set_error("sba_covariance: not available with shared calibration (n_common > 0)"); return SBA_E_INVALID; }
+    const int M = p->M, nc = p->nc, ns = M * nc;
+    const long long n_free = (long long)(M - p->n_cam_fix) * nc + 3LL * (p->N - p->n_pts_fix);
+    const long long dof = 2 * (long long)p->K - n_free;
+    if (!(sigma2 > 0.0) && dof <= 0) {
+        set_error("sba_covariance: " + std::to_string(dof) + " degrees of freedom (2 K - free variables): sigma^2 cannot be estimated");
+        return SBA_E_INVALID;
+    }
+    SBA_CUDA(cudaSetDevice(p->device));
+    cudaStream_t s = p->stream;
+    if (!p->cov_cam) {
+        SBA_TRY(dev_alloc(p, &p->cov_cam, (size_t)ns * ns));
+        SBA_TRY(dev_alloc(p, &p->cov_pts, 6 * (size_t)p->N));
+        SBA_TRY(dev_alloc(p, &p->cov_diag, 4));
+        for (cudaEvent_t& e : p->cov_ev) SBA_CUDA(cudaEventCreate(&e));
+    }
+    const int* tiles = nullptr;
+    int n_tiles = 0;
+    SBA_TRY(cov_tiles(p, &tiles, &n_tiles));
+    // phase 0 starts when x is on the device (the upload from pageable host memory is not device work)
+    SBA_TRY(form_reduced_system(p, x, loss, f_scale, 0.0, p->cov_ev[0]));
+    // the pattern engine's evaluation swapped its buffer sets (pt_accept): swap them back on every exit, so that the handle is
+    // left with the same buffer roles as before the call
+    struct Unswap { sba_problem* p; ~Unswap() { if (p->engine == 1) pt_accept(p); } } unswap{p};
+    // sigma2 estimated: the cost at x by the residual kernel of sba_residuals, in float64 like the Jacobian rows (rpc_float32 is
+    // for fun parity only).  sigma2 given: the assembly's own cost serves the finiteness check.
+    int cost_slot = p->engine == 1 ? SC_COST_NEW : SC_COST;
+    if (!(sigma2 > 0.0)) {
+        cost_slot = SC_SCRATCH;
+        SBA_TRY(run_residual(p, p->x, p->camrec, loss, f_scale, nullptr, SC_SCRATCH, 0));
+    }
+    SBA_CUDA(cudaEventRecord(p->cov_ev[1], s));
+    // factor (frozen slots: identity rows of S) and pivot test
+    SBA_TRY(launch_cholesky_solve(p->S, p->S + (size_t)ns * ns, p->delta, ns, p->scal + SC_CHOL_FAIL, p->chol_work, s, true));
+    p->launches++;
+    SBA_CUDA(cudaMemsetAsync(p->cov_diag, 0, 4 * sizeof(double), s));
+    k_cov_pivots<<<1, 256, 0, s>>>(p->S, p->camsys, ns, nc, p->n_cam_fix, p->scal + SC_CHOL_FAIL, COV_PIVOT_THRESHOLD, p->cov_diag);
+    SBA_TRY(check_launch(p));
+    SBA_CUDA(cudaEventRecord(p->cov_ev[2], s));
+    double* h = p->h_scal + SC_COUNT;            // the slots after the scalar block (used by the PCG path only)
+    SBA_CUDA(cudaMemcpyAsync(h, p->cov_diag, 3 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    SBA_CUDA(cudaMemcpyAsync(p->h_scal + cost_slot, p->scal + cost_slot, sizeof(double), cudaMemcpyDeviceToHost, s));
+    SBA_CUDA(cudaStreamSynchronize(s));
+    const double min_ratio = h[0], cost = p->h_scal[cost_slot];
+    if (min_pivot_ratio_out) *min_pivot_ratio_out = min_ratio;
+    if (h[1] >= 0.0) {
+        const int k = (int)h[1];
+        char msg[256];
+        snprintf(msg, sizeof(msg),
+                 "sba_covariance: the reduced camera system is rank deficient (gauge not fixed?): camera %d, slot %d: pivot ratio "
+                 "L_kk^2 / U_kk = %.3e <= %.0e", k / nc, k % nc, h[2], COV_PIVOT_THRESHOLD);
+        set_error(msg);
+        return SBA_E_NUMERIC;
+    }
+    if (!std::isfinite(cost)) { set_error("sba_covariance: residuals are not finite at x"); return SBA_E_NUMERIC; }
+    const double s2 = sigma2 > 0.0 ? sigma2 : 2.0 * cost / (double)dof;
+    // s2 S^-1, exactly symmetric, frozen rows / columns 0
+    k_cov_inverse<<<(ns + 31) / 32, 256, 0, s>>>(p->S, ns, p->cov_cam);
+    SBA_TRY(check_launch(p));
+    k_cov_finish<<<grid_for((long long)ns * ns, 256, NUM_SMS * 4), 256, 0, s>>>(p->cov_cam, ns, p->n_cam_fix * nc, s2);
+    SBA_TRY(check_launch(p));
+    SBA_CUDA(cudaEventRecord(p->cov_ev[3], s));
+    {
+        const size_t c_bytes = (size_t)ns * ns * sizeof(double);
+        const int in_smem = c_bytes <= COV_SMEM_MAX;
+        const int npf = p->engine == 1 ? p->n_pts_fix_int : p->n_pts_fix;
+        const int* perm = p->engine == 1 ? p->trk_new2old : nullptr;
+        const int grid_long = std::max(1, std::min((n_tiles + 3) / 4, NUM_SMS * 4));
+#define L(MODEL, NC)                                                                                                          \
+    {                                                                                                                         \
+        const size_t smem = ((size_t)COV_WARPS * cov_warp_doubles<NC>() + COV_WARPS * 32 / 2) * sizeof(double) +           \
+                            (in_smem ? c_bytes : 0);                                                                          \
+        SBA_CUDA(cudaFuncSetAttribute(k_cov_points<MODEL, NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));      \
+        const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(8, (size_t)(200 * 1024) / smem));                      \
+        const int grid = std::max(1, std::min((n_tiles + COV_WARPS - 1) / COV_WARPS, NUM_SMS * per_sm));                   \
+        k_cov_points<MODEL, NC><<<grid, COV_THREADS, smem, s>>>(obs_arrays(p), tiles, n_tiles, p->x + (size_t)ns, p->camrec,  \
+                                                               p->rpc_tab, p->n_cam_fix, npf, loss, f_scale, p->cov_cam, ns,   \
+                                                               in_smem, s2, perm, p->cov_pts, p->cov_diag + 3);               \
+        SBA_TRY(check_launch(p));                                                                                             \
+        k_cov_long_tracks<MODEL, NC><<<grid_long, 128, 0, s>>>(obs_arrays(p), tiles, n_tiles, p->x + (size_t)ns, p->camrec,   \
+                                                              p->rpc_tab, p->n_cam_fix, npf, loss, f_scale, p->cov_cam, ns, s2, \
+                                                              perm, p->cov_pts, p->cov_diag + 3);                             \
+    }
+        SBA_DISPATCH(p, L);
+#undef L
+        SBA_TRY(check_launch(p));
+    }
+    SBA_CUDA(cudaEventRecord(p->cov_ev[4], s));
+    if (cov_cam) SBA_CUDA(cudaMemcpyAsync(cov_cam, p->cov_cam, (size_t)ns * ns * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (cov_pts) SBA_CUDA(cudaMemcpyAsync(cov_pts, p->cov_pts, 6 * (size_t)p->N * sizeof(double), cudaMemcpyDeviceToHost, s));
+    SBA_CUDA(cudaMemcpyAsync(h + 3, p->cov_diag + 3, sizeof(double), cudaMemcpyDeviceToHost, s));
+    SBA_CUDA(cudaStreamSynchronize(s));
+    for (int k = 0; k < 4; ++k) {
+        float ms = 0.f;
+        SBA_CUDA(cudaEventElapsedTime(&ms, p->cov_ev[k], p->cov_ev[k + 1]));
+        p->cov_ms[k] = ms;
+    }
+    if (h[3] != 0.0) {
+        set_error("sba_covariance: " + std::to_string((long long)h[3]) + " free point(s) with a singular 3x3 block V_t");
+        return SBA_E_NUMERIC;
+    }
+    if (sigma2_out) *sigma2_out = s2;
+    return SBA_OK;
+}
+
+extern "C" int sba_covariance_phase_ms(const sba_problem* p, double* ms4)
+{
+    if (!p || !ms4) { set_error("null argument"); return SBA_E_INVALID; }
+    for (int k = 0; k < 4; ++k) ms4[k] = p->cov_ms[k];
     return SBA_OK;
 }
 

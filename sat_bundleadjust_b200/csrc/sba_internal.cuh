@@ -177,4 +177,12 @@ struct sba_problem {
     double *osc = nullptr, *osc2 = nullptr;                         // (2K) per-observation robust row scales at the current / trial point
     double *pt_records = nullptr;                                   // Schur records, one per (unit, pass)
     double *r_int = nullptr, *e_int = nullptr;                      // (2K), (K) residuals / errors in internal order
+
+    // ---- posterior covariance (sba_covariance), allocated by its first call ----
+    double *cov_cam = nullptr, *cov_pts = nullptr;                  // (ns x ns) s2 S^-1, (N, 6) point blocks in the caller's order
+    double *cov_diag = nullptr;                                     // pivot test: min ratio, rejected slot, its ratio; bad points
+    int* cov_tile_obs = nullptr;                                    // pattern engine: warp tiles of the point pass (internal order)
+    int cov_n_tiles = 0;
+    cudaEvent_t cov_ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    double cov_ms[4] = {0.0, 0.0, 0.0, 0.0};                        // device time of the phases of the last call
 };

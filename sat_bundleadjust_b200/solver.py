@@ -99,6 +99,7 @@ class DeviceProblem:
         d.n_cam, d.n_pts, d.n_obs = self.n_cam, self.n_pts, self.n_obs
         d.n_params, d.n_cam_params = self.n_params, self._keep[4].shape[1]
         d.n_cam_fix, d.n_pts_fix = int(p.n_cam_fix), int(n_pts_fix)
+        self._n_cam_fix = int(p.n_cam_fix)
         d.cam_ind = self._keep[0].ctypes.data_as(_lib.c_int64_p)
         d.pts_ind = self._keep[1].ctypes.data_as(_lib.c_int64_p)
         d.pts2d, d.pts2d_w, d.cam_params = dptr(self._keep[2]), dptr(self._keep[3]), dptr(self._keep[4])
@@ -191,6 +192,33 @@ class DeviceProblem:
         check(self.lib.sba_reduced_system(self.handle, dptr(x), LOSS_IDS[loss], ctypes.c_double(f_scale), ctypes.c_double(reg),
                                           dptr(S), dptr(rhs)))
         return S, rhs
+
+    def covariance(self, x, loss="linear", f_scale=1.0, sigma2=None):
+        """
+        Posterior covariance at x (sat_bundleadjust_b200.ba_covariance has the definitions): (cov_cam (n_cam n_params)^2,
+        cov_pts (n_pts, 3, 3), sigma2 (given or estimated), min_pivot_ratio).  A rank-deficient reduced camera system (gauge
+        not fixed) or a free point with a singular block raises SbaError.
+        """
+        self._no_common("covariance")
+        n_free = (self.n_cam - self._n_cam_fix) * self.n_params + 3 * (self.n_pts - self._fixed_pts.size // 3)
+        if not (sigma2 is not None and sigma2 > 0) and 2 * self.n_obs - n_free <= 0:
+            raise ValueError("no degrees of freedom left (2 K - n_free = %d): sigma^2 cannot be estimated" % (2 * self.n_obs - n_free))
+        x = self._vars(x)
+        ns = self.n_cam * self.n_params
+        cov_cam = np.empty((ns, ns), order="F")
+        cov6 = np.empty((self.n_pts, 6))
+        s2, ratio = ctypes.c_double(), ctypes.c_double()
+        check(self.lib.sba_covariance(self.handle, dptr(x), LOSS_IDS[loss], ctypes.c_double(f_scale),
+                                      ctypes.c_double(sigma2 if sigma2 is not None else 0.0), dptr(cov_cam), dptr(cov6),
+                                      ctypes.byref(s2), ctypes.byref(ratio)))
+        cov_pts = cov6[:, [0, 1, 2, 1, 3, 4, 2, 4, 5]].reshape(self.n_pts, 3, 3)
+        return cov_cam, cov_pts, s2.value, ratio.value
+
+    def covariance_phase_ms(self):
+        """Device time of the phases of the last covariance call: reduced system, factor + pivot test, inverse, points."""
+        ms = np.zeros(4)
+        check(self.lib.sba_covariance_phase_ms(self.handle, dptr(ms)))
+        return dict(zip(["reduced_system", "factor_pivots", "inverse", "points"], ms.tolist()))
 
     @staticmethod
     def make_opts(loss="linear", f_scale=1.0, ftol=1e-4, xtol=1e-10, gtol=1e-8, max_nfev=300, verbose=0,
