@@ -565,30 +565,142 @@ static int run_gauss_newton_step(sba_problem* p, int loss, double f_scale, Phase
 }
 
 
+#include "sba_pattern_host.inl"
+
 // ------------------------------------------------------------------------------------------------
-// the iteration
+// the iteration: one driver for both engines, which differ only in the launch sequences below
 // ------------------------------------------------------------------------------------------------
-static int solve_on_device(sba_problem* p, const sba_solve_opts* o, sba_solve_info* info)
+// state of a fresh solve from the start vector in p->x
+static int trf_reset(sba_problem* p)
+{
+    if (p->engine == 1) return pt_reset_state(p);
+    SBA_CUDA(cudaMemsetAsync(p->scal, 0, SC_COUNT * sizeof(double), p->stream));
+    return SBA_OK;
+}
+
+// the cost at x0 into scal[SC_COST_NEW], by the same kernels as every later trial point
+static int trf_cost_x0(sba_problem* p, const sba_solve_opts* o)
+{
+    if (p->engine == 1) return pt_run_assemble(p, 1, 1, o->loss, o->f_scale);
+    SBA_TRY(run_prepare(p, p->x, p->camrec));
+    SBA_TRY(run_residual(p, p->x, p->camrec, o->loss, o->f_scale, nullptr, SC_COST_NEW, 0));
+    return allreduce_scal(p, SC_COST_NEW, 1);
+}
+
+// the blocks at x0 (the pattern engine's cost evaluation has computed them already)
+static int trf_blocks_x0(sba_problem* p, const sba_solve_opts* o)
+{
+    if (p->engine == 1) { pt_accept(p); return SBA_OK; }
+    return run_assemble(p, p->x, p->camrec, o->loss, o->f_scale);
+}
+
+// everything from the blocks at x to the scalars of the 2-D subproblem, with no host round trip.
+// reg_override >= 0: re-damp the system of this iteration with that value
+static int trf_step(sba_problem* p, const sba_solve_opts* o, PhaseTimer& tm, bool first, double Delta, double reg_override)
 {
     const int loss = o->loss;
     const double fs = o->f_scale;
     const int ns = p->M * p->nc;
+    if (p->engine == 1) {
+        if (reg_override < 0.0) {
+            tm.begin(SBA_PH_SCALE_JVP);
+            SBA_TRY(pt_run_jvp1(p, first ? 1 : 0, loss, fs, Delta));       // and the damping
+            tm.end();
+        } else {
+            k_control_reg<<<1, 32, 0, p->stream>>>(p->scal, Delta, reg_override);
+            SBA_TRY(check_launch(p));
+        }
+        tm.begin(SBA_PH_SCHUR);
+        SBA_TRY(pt_run_schur(p, loss, fs));
+        tm.end();
+        tm.begin(SBA_PH_CHOLESKY);
+        SBA_TRY(launch_cholesky_solve(p->S, p->S + (size_t)ns * ns, p->delta, ns, p->scal + SC_CHOL_FAIL, p->chol_work, p->stream, false));
+        p->launches++;
+        tm.end();
+        tm.begin(SBA_PH_BACKSUB);
+        SBA_TRY(pt_run_backsub(p, loss, fs));
+        tm.end();
+        return SBA_OK;
+    }
     const int elem_grid = grid_for(p->n, 256, NUM_SMS * 8);
+    if (reg_override < 0.0) {
+        tm.begin(SBA_PH_SCALE_JVP);
+        SBA_TRY(run_scale_dots(p, first ? 1 : 0));
+        Slots sa; sa.s[0] = SC_A; sa.s[1] = SC_SCRATCH; sa.s[2] = SC_SCRATCH;
+        SBA_TRY(run_jvp(p, loss, fs, 1, sa));
+        SBA_TRY(allreduce_scal(p, SC_COST, SC_GGN - SC_COST));
+        tm.end();
+    }
+    k_control_reg<<<1, 32, 0, p->stream>>>(p->scal, Delta, reg_override);
+    SBA_TRY(check_launch(p));
+    SBA_TRY(run_gauss_newton_step(p, loss, fs, tm));
+    tm.begin(SBA_PH_SUBSPACE);
+    k_dot_g_delta<<<elem_grid, 256, 0, p->stream>>>(p->g, p->sinv, p->delta, p->n, ns, p->rank == 0, p->red_partials,
+                                                    p->counters + 4, p->scal);
+    SBA_TRY(check_launch(p));
+    SBA_TRY(allreduce_scal(p, SC_GGN, 2));
+    k_build_t2<<<elem_grid, 256, 0, p->stream>>>(p->g, p->sinv, p->delta, p->t1, p->t2, p->n, ns, p->rank == 0,
+                                                 p->red_partials, p->counters + 5, p->scal);
+    SBA_TRY(check_launch(p));
+    Slots sb; sb.s[0] = SC_B11; sb.s[1] = SC_B12; sb.s[2] = SC_B22;
+    SBA_TRY(run_jvp(p, loss, fs, 2, sb));
+    SBA_TRY(allreduce_scal(p, SC_WW, 8));      // [ww wg t11 t12 t22 | b11 b12 b22] in one exchange
+    tm.end();
+    return SBA_OK;
+}
+
+// trial point x_new = x + c1 t1 + c2 t2 for radius `radius` (< 0: the one on the device) and its cost into scal[SC_COST_NEW]
+static int trf_trial(sba_problem* p, const sba_solve_opts* o, double radius)
+{
+    if (p->engine == 1) {
+        if (radius >= 0.0) {        // else K4 has solved the 2-D subproblem already
+            k_pt_control_tr2d<<<1, 32, 0, p->stream>>>(p->scal, radius);
+            SBA_TRY(check_launch(p));
+        }
+        return pt_run_assemble(p, 0, 0, o->loss, o->f_scale);     // K1: the cost, and the blocks should x_new be accepted
+    }
+    k_control_tr2d<<<1, 32, 0, p->stream>>>(p->scal, radius);
+    SBA_TRY(check_launch(p));
+    k_step<<<grid_for(p->n, 256, NUM_SMS * 8), 256, 0, p->stream>>>(p->x, p->t1, p->t2, p->scal, p->x_new, p->n, p->cam_static,
+                                                                    p->camrec_new, p->M, p->P, p->nc, p->n_cam_fix, p->n_common,
+                                                                    p->model);
+    SBA_TRY(check_launch(p));
+    SBA_TRY(run_residual(p, p->x_new, p->camrec_new, o->loss, o->f_scale, nullptr, SC_COST_NEW, 0));
+    return allreduce_scal(p, SC_COST_NEW, 1);
+}
+
+// the trial point becomes the current point; its blocks are needed unless the solve terminates
+static int trf_accept(sba_problem* p, const sba_solve_opts* o, PhaseTimer& tm, bool terminating, int& njev)
+{
+    if (p->engine == 1) {
+        pt_accept(p);               // the trial evaluation already holds the blocks of the new point
+        ++njev;
+        return SBA_OK;
+    }
+    std::swap(p->x, p->x_new);
+    std::swap(p->camrec, p->camrec_new);
+    if (terminating) return SBA_OK;
+    tm.begin(SBA_PH_ASSEMBLE);
+    SBA_TRY(run_assemble(p, p->x, p->camrec, o->loss, o->f_scale));
+    tm.end();
+    ++njev;
+    return SBA_OK;
+}
+
+static int solve_trf(sba_problem* p, const sba_solve_opts* o, sba_solve_info* info)
+{
     std::memset(info, 0, sizeof(*info));
     if (o->max_nfev < 1) { set_error("max_nfev must be >= 1"); return SBA_E_INVALID; }
     p->launches = 0;
     p->pcg_iterations = 0; p->pcg_solves = 0;
-    SBA_CUDA(cudaMemsetAsync(p->scal, 0, SC_COUNT * sizeof(double), p->stream));
+    SBA_TRY(trf_reset(p));
     SBA_CUDA(cudaEventRecord(p->ev0, p->stream));
-
-    SBA_TRY(run_prepare(p, p->x, p->camrec));
-    SBA_TRY(run_residual(p, p->x, p->camrec, loss, fs, nullptr, SC_COST_NEW, 0));   // cost at x0, same kernel as every later cost
-    SBA_TRY(allreduce_scal(p, SC_COST_NEW, 1));
+    SBA_TRY(trf_cost_x0(p, o));
     SBA_TRY(fetch_scal(p));
     double cost = p->h_scal[SC_COST_NEW];
     if (!std::isfinite(cost)) { set_error("Residuals are not finite in the initial point."); return SBA_E_NUMERIC; }
     info->cost_init = cost;
-    SBA_TRY(run_assemble(p, p->x, p->camrec, loss, fs));
+    SBA_TRY(trf_blocks_x0(p, o));
     int nfev = 1, njev = 1, iteration = 0, status = -1, chol_retries = 0;
     double Delta = -1.0, g_norm = 0.0;   // Delta < 0: not initialised yet (the device sets |x0 * scale_inv|)
     bool first = true;
@@ -601,45 +713,18 @@ static int solve_on_device(sba_problem* p, const sba_solve_opts* o, sba_solve_in
         SBA_CUDA(cudaMalloc(&p->flush_buf, (size_t)o->l2_flush_bytes));
         p->flush_bytes = (size_t)o->l2_flush_bytes;
     }
+    // scalars of the 2-D subproblem that are not finite when the damped system had no usable solution
+    const int chk0 = p->engine == 1 ? SC_P_GD : SC_GGN, chk1 = p->engine == 1 ? SC_P_C22 : SC_B22;
 
-    // enqueue: trial point x_new = x + c1 t1 + c2 t2 for radius `radius` (< 0: the one on the device) and its cost
     auto enqueue_trial = [&](double radius) -> int {
         tm.begin(SBA_PH_STEP_EVAL);
-        k_control_tr2d<<<1, 32, 0, p->stream>>>(p->scal, radius);
-        SBA_TRY(check_launch(p));
-        k_step<<<elem_grid, 256, 0, p->stream>>>(p->x, p->t1, p->t2, p->scal, p->x_new, p->n, p->cam_static,
-                                                 p->camrec_new, p->M, p->P, p->nc, p->n_cam_fix, p->n_common, p->model);
-        SBA_TRY(check_launch(p));
-        SBA_TRY(run_residual(p, p->x_new, p->camrec_new, loss, fs, nullptr, SC_COST_NEW, 0));
-        SBA_TRY(allreduce_scal(p, SC_COST_NEW, 1));
+        SBA_TRY(trf_trial(p, o, radius));
         tm.end();
         return SBA_OK;
     };
-    // enqueue: everything from the Jacobian blocks at x to the first trial point, with no host round trip
+    // everything from the blocks at x to the first trial point
     auto enqueue_iteration = [&](double reg_override) -> int {
-        if (reg_override < 0.0) {
-            tm.begin(SBA_PH_SCALE_JVP);
-            SBA_TRY(run_scale_dots(p, first ? 1 : 0));
-            Slots sa; sa.s[0] = SC_A; sa.s[1] = SC_SCRATCH; sa.s[2] = SC_SCRATCH;
-            SBA_TRY(run_jvp(p, loss, fs, 1, sa));
-            SBA_TRY(allreduce_scal(p, SC_COST, SC_GGN - SC_COST));
-            tm.end();
-        }
-        k_control_reg<<<1, 32, 0, p->stream>>>(p->scal, Delta, reg_override);
-        SBA_TRY(check_launch(p));
-        SBA_TRY(run_gauss_newton_step(p, loss, fs, tm));
-        tm.begin(SBA_PH_SUBSPACE);
-        k_dot_g_delta<<<elem_grid, 256, 0, p->stream>>>(p->g, p->sinv, p->delta, p->n, ns, p->rank == 0, p->red_partials,
-                                                        p->counters + 4, p->scal);
-        SBA_TRY(check_launch(p));
-        SBA_TRY(allreduce_scal(p, SC_GGN, 2));
-        k_build_t2<<<elem_grid, 256, 0, p->stream>>>(p->g, p->sinv, p->delta, p->t1, p->t2, p->n, ns, p->rank == 0,
-                                                     p->red_partials, p->counters + 5, p->scal);
-        SBA_TRY(check_launch(p));
-        Slots sb; sb.s[0] = SC_B11; sb.s[1] = SC_B12; sb.s[2] = SC_B22;
-        SBA_TRY(run_jvp(p, loss, fs, 2, sb));
-        SBA_TRY(allreduce_scal(p, SC_WW, 8));      // [ww wg t11 t12 t22 | b11 b12 b22] in one exchange
-        tm.end();
+        SBA_TRY(trf_step(p, o, tm, first, Delta, reg_override));
         return enqueue_trial(-1.0);
     };
 
@@ -657,7 +742,7 @@ static int solve_on_device(sba_problem* p, const sba_solve_opts* o, sba_solve_in
         SBA_TRY(fetch_scal(p));
         const double* h = p->h_scal;
         if (h[SC_COMM_FAIL] != 0.0) { set_error("peer-memory all-reduce timed out (a rank is missing)"); return SBA_E_CUDA; }
-        for (int attempt = 0; h[SC_CHOL_FAIL] != 0.0 || !std::isfinite(h[SC_GGN]) || !std::isfinite(h[SC_B22]); ++attempt) {
+        for (int attempt = 0; h[SC_CHOL_FAIL] != 0.0 || !std::isfinite(h[chk0]) || !std::isfinite(h[chk1]); ++attempt) {
             if (attempt >= 30) { set_error("reduced camera system could not be factorised"); return SBA_E_NUMERIC; }
             // re-damp: J_h has unit column norms, so reg is relative to 1
             ++chol_retries;
@@ -675,51 +760,26 @@ static int solve_on_device(sba_problem* p, const sba_solve_opts* o, sba_solve_in
                    h[SC_REG]);
         if (g_norm < o->gtol) { status = 1; break; }
 
-        double actual_reduction = -1.0, cost_new = cost;
-        int term = -1;
+        double cost_new;
+        TrOutcome tr;
         while (true) {
             ++nfev;
             cost_new = h[SC_COST_NEW];
-            const double predicted = h[SC_PRED], step_h_norm = h[SC_STEPH], step_norm = h[SC_STEPN];
-            if (!std::isfinite(cost_new)) {
-                Delta = 0.25 * step_h_norm;
-            } else {
-                actual_reduction = cost - cost_new;
-                // update_tr_radius (common.py:222-245)
-                double ratio;
-                if (predicted > 0.0) ratio = actual_reduction / predicted;
-                else if (predicted == 0.0 && actual_reduction == 0.0) ratio = 1.0;
-                else ratio = 0.0;
-                double Delta_new = Delta;
-                if (ratio < 0.25) Delta_new = 0.25 * step_h_norm;
-                else if (ratio > 0.75 && step_h_norm > 0.95 * Delta) Delta_new = 2.0 * Delta;
-                // check_termination (common.py:705-717)
-                const bool ftol_ok = actual_reduction < o->ftol * cost && ratio > 0.25;
-                const bool xtol_ok = step_norm < o->xtol * (o->xtol + x_norm);
-                if (ftol_ok && xtol_ok) term = 4; else if (ftol_ok) term = 2; else if (xtol_ok) term = 3;
-                if (term >= 0) break;
-                Delta = Delta_new;
-            }
-            if (actual_reduction > 0.0 || nfev >= o->max_nfev) break;
+            tr = tr_outcome(cost, cost_new, h[SC_PRED], h[SC_STEPH], h[SC_STEPN], x_norm, Delta, o->ftol, o->xtol);
+            Delta = tr.Delta;
+            if (tr.accept || tr.status >= 0 || nfev >= o->max_nfev) break;
             // rejected: same model, smaller radius, new trial point (no new factorisation, like scipy)
             SBA_TRY(enqueue_trial(Delta));
             SBA_TRY(fetch_scal(p));
             h = p->h_scal;
         }
-        if (actual_reduction > 0.0) {
-            std::swap(p->x, p->x_new);
-            std::swap(p->camrec, p->camrec_new);
+        if (tr.accept) {
             cost = cost_new;
-            if (term < 0) {
-                tm.begin(SBA_PH_ASSEMBLE);
-                SBA_TRY(run_assemble(p, p->x, p->camrec, loss, fs));
-                tm.end();
-                ++njev;
-            }
+            SBA_TRY(trf_accept(p, o, tm, tr.status >= 0, njev));
         }
         it_tm.end();
         ++iteration;
-        if (term >= 0) { status = term; break; }
+        if (tr.status >= 0) { status = tr.status; break; }
     }
     if (status < 0) status = 0;
     SBA_CUDA(cudaEventRecord(p->ev1, p->stream));
@@ -735,8 +795,6 @@ static int solve_on_device(sba_problem* p, const sba_solve_opts* o, sba_solve_in
     it_tm.resolve(info);
     return SBA_OK;
 }
-
-#include "sba_pattern_host.inl"
 
 // residuals at the internal vector x (camrec prepared) into a device buffer in the CALLER's observation order
 static int residuals_ext(sba_problem* p, const double* x, const double* camrec, int loss, double f_scale, double* r_ext_dev,
@@ -1274,7 +1332,7 @@ static int form_reduced_system(sba_problem* p, const double* x, int32_t loss, do
         SBA_TRY(pt_run_assemble(p, 1, 1, loss, f_scale));
         pt_accept(p);
         SBA_TRY(pt_run_jvp1(p, 1, loss, f_scale, -1.0));
-        k_pt_control_reg<<<1, 32, 0, p->stream>>>(p->scal, -1.0, reg);
+        k_control_reg<<<1, 32, 0, p->stream>>>(p->scal, -1.0, reg);
         SBA_TRY(check_launch(p));
         SBA_TRY(pt_run_schur(p, loss, f_scale));
     } else {
@@ -1463,8 +1521,7 @@ extern "C" int sba_solve_device(sba_problem* p, const double* x0_dev, const sba_
     if (p->world > 1 && !p->allreduce && !p->comm_ready) { set_error("world_size > 1 needs sba_comm_import or sba_problem_set_allreduce"); return SBA_E_INVALID; }
     SBA_CUDA(cudaSetDevice(p->device));
     SBA_TRY(vars_in(p, x0_dev, p->x));
-    if (p->engine == 1) SBA_TRY(solve_pattern(p, opts, info));
-    else SBA_TRY(solve_on_device(p, opts, info));
+    SBA_TRY(solve_trf(p, opts, info));
     if (x_dev) SBA_TRY(vars_out(p, p->x, x_dev));
     if (r_dev) {
         SBA_TRY(residuals_ext(p, p->x, p->camrec, SBA_LOSS_LINEAR, 1.0, r_dev, SC_SCRATCH, p->rpc_f32));

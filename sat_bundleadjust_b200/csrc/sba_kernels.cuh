@@ -1089,10 +1089,10 @@ k_step(const double* __restrict__ x, const double* __restrict__ t1, const double
 // already reduced scalars, so that the host reads the scalar block once per trial step instead of three times
 // ------------------------------------------------------------------------------------------------
 // damping from the Cauchy step (scipy trf.py:485-490): reg = -min_{0<=t<=Delta/|g_h|} (a t^2 + b t) / Delta^2
-// delta_arg < 0: first iteration, Delta = |x0 * scale_inv| (or 1);  reg_override >= 0: use that value (re-damping)
-__global__ void k_control_reg(double* scal, double delta_arg, double reg_override)
+// delta_arg < 0: first iteration, Delta = |x0 * scale_inv| (or 1);  reg_override >= 0: use that value (re-damping).
+// Also run in the epilogue of the pattern engine's K2 (k_pt_jvp1).
+__device__ __forceinline__ void control_reg_dev(double* scal, double delta_arg, double reg_override)
 {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
     double Delta = delta_arg;
     if (Delta < 0.0) {
         Delta = sqrt(scal[SC_XS]);
@@ -1110,6 +1110,11 @@ __global__ void k_control_reg(double* scal, double delta_arg, double reg_overrid
         if (ext > 0.0 && ext < to_tr) ag = fmin(ag, ext * (qa * ext + qb));
     }
     scal[SC_REG] = -ag / (Delta * Delta);
+}
+
+__global__ void k_control_reg(double* scal, double delta_arg, double reg_override)
+{
+    if (threadIdx.x == 0 && blockIdx.x == 0) control_reg_dev(scal, delta_arg, reg_override);
 }
 
 // exact 2-D trust-region step in span{g_h, gn_h} (scipy trf.py:496-509) for the radius `delta_arg`

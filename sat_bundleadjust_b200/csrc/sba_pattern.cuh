@@ -431,29 +431,9 @@ k_pt_cam_scale(const double* __restrict__ camsys, const double* __restrict__ dsq
 }
 
 // ------------------------------------------------------------------------------------------------
-// device-side control (shared by the single-thread kernels and the folded epilogues)
+// device-side control (shared by the single-thread kernel and the folded epilogue; the damping rule control_reg_dev is
+// in sba_kernels.cuh, shared with the generic engine)
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void control_reg_dev(double* scal, double delta_arg, double reg_override)
-{
-    double Delta = delta_arg;
-    if (Delta < 0.0) {
-        Delta = sqrt(scal[SC_XS]);
-        if (Delta == 0.0) Delta = 1.0;
-    }
-    scal[SC_DELTA] = Delta;
-    if (reg_override >= 0.0) { scal[SC_REG] = reg_override; return; }
-    const double gg = scal[SC_GG];
-    const double qa = 0.5 * scal[SC_A], qb = -gg;
-    const double to_tr = Delta / sqrt(gg);
-    double ag = 0.0;
-    ag = fmin(ag, to_tr * (qa * to_tr + qb));
-    if (qa != 0.0) {
-        const double ext = -0.5 * qb / qa;
-        if (ext > 0.0 && ext < to_tr) ag = fmin(ag, ext * (qa * ext + qb));
-    }
-    scal[SC_REG] = -ag / (Delta * Delta);
-}
-
 // 2-D subspace {g_h, gn_h}: the Gram scalars of (t1, delta) are turned into those of the orthogonalised pair (t1, t2 = delta -
 // alpha t1), then the exact 2-D trust-region problem is solved (scipy trf.py:496-509).  Step = pa t1 + pb delta.
 __device__ __forceinline__ void control_tr2d_gram_dev(double* scal, double delta_arg)
@@ -485,10 +465,6 @@ __device__ __forceinline__ void control_tr2d_gram_dev(double* scal, double delta
     scal[SC_B22] = b22;                                // diagnostics read by the host
 }
 
-__global__ void k_pt_control_reg(double* scal, double delta_arg, double reg_override)
-{
-    if (threadIdx.x == 0 && blockIdx.x == 0) control_reg_dev(scal, delta_arg, reg_override);
-}
 __global__ void k_pt_control_tr2d(double* scal, double delta_arg)
 {
     if (threadIdx.x == 0 && blockIdx.x == 0) control_tr2d_gram_dev(scal, delta_arg);

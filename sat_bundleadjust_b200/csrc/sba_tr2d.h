@@ -3,7 +3,8 @@
 // is positive definite and the step is inside the region, otherwise the global minimiser on the
 // boundary.  scipy finds the boundary minimiser through the roots of a quartic (numpy.roots); here it
 // is found from the 2x2 eigen-decomposition and the secular equation, which has no LAPACK dependency
-// and runs unchanged on the device.
+// and runs unchanged on the device.  Below it, the rule that turns one evaluated trial point into the next radius,
+// a termination code and the accept/reject decision.
 #pragma once
 #include <math.h>
 
@@ -83,6 +84,37 @@ SBA_HD bool solve_trust_region_2d(double b00, double b01, double b11, double g0,
     if (nn > 0.0) { p1 *= Delta / nn; p2 *= Delta / nn; }
     p[0] = -s_ * p1 + c * p2; p[1] = c * p1 + s_ * p2;
     return false;
+}
+
+// What one evaluated trial point does to the trust-region iteration: scipy's trf_no_bounds inner loop (trf.py:511-560)
+// with update_tr_radius (common.py:222-245) and check_termination (common.py:705-717).  A non-finite cost_new shrinks
+// the radius to |step_h| / 4 and is neither tested for termination nor accepted; the radius is kept when a termination
+// test fires; the step is accepted iff it reduces the cost.
+struct TrOutcome {
+    double Delta;     // radius of the next trial point
+    int status;       // termination: 2 ftol, 3 xtol, 4 both, -1 none
+    bool accept;
+};
+
+SBA_HD TrOutcome tr_outcome(double cost, double cost_new, double predicted, double step_h_norm, double step_norm,
+                            double x_norm, double Delta, double ftol, double xtol)
+{
+    TrOutcome r = {Delta, -1, false};
+    if (!isfinite(cost_new)) { r.Delta = 0.25 * step_h_norm; return r; }
+    const double actual = cost - cost_new;
+    double ratio;
+    if (predicted > 0.0) ratio = actual / predicted;
+    else if (predicted == 0.0 && actual == 0.0) ratio = 1.0;
+    else ratio = 0.0;
+    const bool ftol_ok = actual < ftol * cost && ratio > 0.25;
+    const bool xtol_ok = step_norm < xtol * (xtol + x_norm);
+    if (ftol_ok && xtol_ok) r.status = 4; else if (ftol_ok) r.status = 2; else if (xtol_ok) r.status = 3;
+    if (r.status < 0) {
+        if (ratio < 0.25) r.Delta = 0.25 * step_h_norm;
+        else if (ratio > 0.75 && step_h_norm > 0.95 * Delta) r.Delta = 2.0 * Delta;
+    }
+    r.accept = actual > 0.0;
+    return r;
 }
 
 }  // namespace sba

@@ -71,6 +71,16 @@ int hh_tr2d(const double* B, const double* g, double Delta, double* p)
     return solve_trust_region_2d(B[0], B[1], B[3], g[0], g[1], Delta, p) ? 1 : 0;
 }
 
+// one evaluated trial point (csrc/sba_tr2d.h tr_outcome): returns the termination code, -1 for none
+int hh_tr_outcome(double cost, double cost_new, double predicted, double step_h_norm, double step_norm, double x_norm,
+                  double Delta, double ftol, double xtol, double* Delta_out, int* accept)
+{
+    const TrOutcome r = tr_outcome(cost, cost_new, predicted, step_h_norm, step_norm, x_norm, Delta, ftol, xtol);
+    *Delta_out = r.Delta;
+    *accept = r.accept ? 1 : 0;
+    return r.status;
+}
+
 // host index construction of a problem (csrc/sba_index.h): sizes first (pass NULL outputs), then the arrays
 int hh_host_index(const long long* cam_ind, const long long* pts_ind, long long K, int M, int N, int chunk, int max_threads,
                   int* sizes /* [n_chunks, n_tiles+1] */, int* cam, int* pts, int* track_ptr, int* cam_cnt, int* cm_obs,

@@ -159,6 +159,70 @@ def test_tr2d_matches_scipy(built):
         assert np.linalg.norm(p1) <= D * (1 + 1e-12)
 
 
+def _scipy_tr_outcome(cost, cost_new, predicted, step_h_norm, step_norm, x_norm, Delta, ftol, xtol):
+    """One trial point of scipy's trf_no_bounds inner loop (trf.py:511-560): (next Delta, termination code, accepted)."""
+    from scipy.optimize._lsq.common import check_termination, update_tr_radius
+    if not np.isfinite(cost_new):
+        return 0.25 * step_h_norm, None, False
+    actual = cost - cost_new
+    Delta_new, ratio = update_tr_radius(Delta, actual, predicted, step_h_norm, step_h_norm > 0.95 * Delta)
+    term = check_termination(actual, cost, step_norm, x_norm, ratio, ftol, xtol)
+    return (Delta if term is not None else Delta_new), term, actual > 0
+
+
+def _tr_outcome_cases():
+    rng = np.random.default_rng(0)
+    cases = []
+    for _ in range(4000):
+        cost = 10 ** rng.uniform(-3, 3)
+        predicted = cost * 10 ** rng.uniform(-8, 0) * rng.choice([1.0, 1.0, 1.0, -1.0, 0.0])
+        ratio = rng.choice([rng.uniform(-1.0, 2.0), 0.25, 0.75, 1.0])
+        actual = ratio * predicted if predicted != 0.0 else cost * rng.choice([0.0, 1e-3, -1e-3])
+        Delta = 10 ** rng.uniform(-3, 3)
+        step_h = Delta * rng.choice([rng.uniform(0.0, 1.0), 0.95, 1.0])
+        x_norm = 10 ** rng.uniform(-2, 4)
+        ftol = rng.choice([1e-4, 1e-8, 10 ** rng.uniform(-8, 0)])
+        xtol = rng.choice([1e-10, 0.0, 10 ** rng.uniform(-10, -1)])
+        step = xtol * (xtol + x_norm) * rng.choice([rng.uniform(0.5, 1.5), 1.0]) if rng.random() < 0.3 else step_h * x_norm
+        cases.append((cost, cost - actual, predicted, step_h, step, x_norm, Delta, ftol, xtol))
+    # the edges of every branch, each against a few radii, step lengths and tolerances
+    edges = [(10.0, 10.0, 0.0),              # predicted = 0, actual = 0: ratio 1
+             (10.0, 9.0, 0.0), (10.0, 11.0, 0.0),   # predicted = 0, actual != 0: ratio 0
+             (10.0, 9.0, -1.0), (10.0, 11.0, -1.0),  # predicted < 0
+             (10.0, 9.0, 4.0), (10.0, 7.0, 4.0),    # ratio exactly 0.25 and 0.75
+             (1.0, 0.75, 0.5), (1.0, 0.75, 0.3),    # dF exactly ftol F (ftol = 0.25 below), ratio 0.5 and 0.83
+             (10.0, np.inf, 1.0), (10.0, np.nan, 1.0), (10.0, -np.inf, 1.0)]
+    for cost, cost_new, predicted in edges:
+        for Delta in (1.0, 3.0):
+            for step_h in (0.5 * Delta, 0.95 * Delta, Delta):
+                for ftol, xtol, x_norm, step in ((0.25, 0.0, 1.0, 0.0), (1e-8, 0.0, 5.0, 1e-3), (1e-8, 0.5, 1.5, 1.0),
+                                                 (1e-8, 0.5, 1.5, 0.999), (0.25, 0.5, 1.5, 0.5)):
+                    cases.append((cost, cost_new, predicted, step_h, step, x_norm, Delta, ftol, xtol))
+    return cases
+
+
+def test_trf_update_matches_scipy(built):
+    """The trust-region update of one trial point (csrc/sba_tr2d.h tr_outcome, run by the solver after every trial
+    point) equals scipy's update_tr_radius + check_termination as trf_no_bounds composes them, bit for bit."""
+    lib = _harness()
+    f = lib.hh_tr_outcome
+    f.restype = ctypes.c_int
+    f.argtypes = [ctypes.c_double] * 9 + [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_int)]
+    seen = set()
+    for c in _tr_outcome_cases():
+        D, acc = ctypes.c_double(), ctypes.c_int()
+        term = f(*c, ctypes.byref(D), ctypes.byref(acc))
+        D0, term0, acc0 = _scipy_tr_outcome(*c)
+        assert (term if term >= 0 else None) == term0, c
+        assert D.value == D0, (c, D.value, D0)
+        assert bool(acc.value) == bool(acc0), c
+        seen.add((term, bool(acc.value), D.value < c[6], D.value > c[6]))
+    # every outcome is exercised: each termination code, accepted and rejected steps, shrinking and growing radii
+    assert {t for t, _, _, _ in seen} == {-1, 2, 3, 4}
+    assert {(a, s, g) for t, a, s, g in seen if t < 0} >= {(True, True, False), (True, False, True), (True, False, False),
+                                                           (False, True, False)}
+
+
 def test_no_cpu_fallback(built):
     """Without a CUDA device the product path must raise, not compute on the CPU."""
     import torch
