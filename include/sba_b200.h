@@ -92,7 +92,7 @@ typedef struct sba_solve_info {
     int32_t status;           /* scipy status: 0 max_nfev, 1 gtol, 2 ftol, 3 xtol, 4 ftol+xtol */
     int32_t nfev, njev;       /* residual evaluations / Jacobian (assembly) evaluations */
     int32_t iterations;       /* outer trust-region iterations */
-    double cost_init, cost;   /* 0.5 * sum(rho) at x0 and at the solution */
+    double cost_init, cost;   /* 0.5 * sum(rho) (+ the camera prior's term) at x0 and at the solution */
     double optimality;        /* ||J^T f||_inf at the solution */
     double solve_ms;          /* device time of the iteration loop (CUDA events) */
     int32_t chol_retries;     /* times the reduced camera system had to be re-damped */
@@ -130,6 +130,17 @@ int sba_comm_import(sba_problem *p, const void *handles_world_x_64_bytes);
 /* Attach to the exchange buffers this process already shares with the same peers (kept across problems: mapping them
  * costs ~15 ms).  Returns 1 when attached, 0 when the export / gather / import sequence is needed. */
 int sba_comm_try_reuse(sba_problem *p);
+/* Gaussian prior on the camera variables (the standard zero-mean weighted constraint of RPC bias compensation, or any
+ * camera knowledge with an accuracy).  mean (n_cam, n_params) in the params_opt camera layout, info (n_cam, n_params,
+ * n_params) symmetric positive semi-definite information matrices L_j.  The solver then minimises
+ *     0.5 f_scale^2 sum_k rho(|r_k|^2 / f_scale^2) + 0.5 sum_{j free} (x_j - mu_j)^T L_j (x_j - mu_j),
+ * i.e. scipy's least_squares on the augmented residual [r ; C_j (x_j - mu_j)] (L_j = C_j^T C_j) with the loss on the
+ * observation rows only: the scaling D, the damping, the steps and every termination test are those of the augmented
+ * problem.  A zero block (row / column) means no prior on that camera (parameter); blocks of frozen cameras are ignored.
+ * Checked on the host: finite values, symmetry to 1e-12 of max|L_j| (then symmetrised), eigenvalues >= -1e-12 of the
+ * largest.  mean = info = NULL clears the prior.  SBA_E_INVALID with n_common > 0.  Applies to the following solves,
+ * sba_normal_blocks, sba_reduced_system and sba_covariance of this handle (in a multi-GPU solve every rank sets the same). */
+int sba_problem_set_camera_prior(sba_problem *p, const double *mean, const double *info);
 /* number of variables n = n_cam * n_params + 3 * n_pts */
 int64_t sba_problem_num_vars(const sba_problem *p);
 /* Which of the two device engines serves this problem (diagnostics / measurement): 1 = pattern-major (reduced camera
@@ -140,19 +151,21 @@ int sba_problem_engine(const sba_problem *p);
 int sba_problem_solver(const sba_problem *p);
 
 /* Replaces ba_core.fun(v, p) (ba_core.py:157-183): x (n) -> weighted residuals r (2K), interleaved.
- * Also returns 0.5*sum(rho(r)) for the given loss in *cost (may be NULL). */
+ * Also returns 0.5*sum(rho(r)) for the given loss in *cost (may be NULL).  Observation rows only: a camera prior adds
+ * neither rows to r nor its term to *cost. */
 int sba_residuals(sba_problem *p, const double *x, double *r, int32_t loss, double f_scale, double *cost);
 
 /* Jacobian pieces at x for tests: per-observation camera block (K,2,n_params), point block (K,2,3),
  * both including observation weights but NOT the robust rescale.  Any output may be NULL. */
 int sba_jacobian_blocks(sba_problem *p, const double *x, double *Jc, double *Jp);
 
-/* Normal-equation blocks at x (robust rescale applied): U (M,c,c), V (N,6: xx xy xz yy yz zz), g (n). */
+/* Normal-equation blocks at x (robust rescale applied): U (M,c,c), V (N,6: xx xy xz yy yz zz), g (n), exactly as the solver
+ * forms them: with a camera prior U_j includes L_j and g its L_j (x_j - mu_j). */
 int sba_normal_blocks(sba_problem *p, const double *x, int32_t loss, double f_scale, double *U, double *V, double *g);
 
 /* The reduced camera system of the damped normal equations at x exactly as the solver forms it (scaling D taken from
  * this one evaluation; shared calibration folded, see n_common): S = U + reg D_c^2 - W (V + reg D_p^2)^-1 W^T,
- * rhs = -(g_c - W (V + reg D_p^2)^-1 g_p).  For the parity tests of the Schur complement (there is no reference
+ * rhs = -(g_c - W (V + reg D_p^2)^-1 g_p), with U, g_c and D including a camera prior.  For the parity tests of the Schur complement (there is no reference
  * counterpart: the reference never forms S).  Host buffers; S is (n_cam n_params)^2, column-major. */
 int sba_reduced_system(sba_problem *p, const double *x, int32_t loss, double f_scale, double reg, double *S, double *rhs);
 
@@ -163,12 +176,15 @@ int sba_reduced_system(sba_problem *p, const double *x, int32_t loss, double f_s
  * J is the Jacobian of the weighted residuals at x over the free variables, rescaled for the robust loss like the solver does
  * (scipy's scale_for_robust_loss_function); H = J^T J = [[U, W], [W^T, V]], S = U - W V^-1 W^T.  cov_cam = sigma2 S^-1 (rows
  * and columns of frozen cameras 0); cov_pts[t] = sigma2 (V_t^-1 + V_t^-1 W_t^T S^-1 W_t V_t^-1) as xx xy xz yy yz zz (frozen
- * points 0).  Estimated sigma2 = 2 cost(x) / (2K - n_free) (scipy curve_fit's convention).  S is rejected as rank deficient
+ * points 0).  Estimated sigma2 = 2 cost(x) / (2K + sum_{j free} rank(L_j) - n_free) (scipy curve_fit's convention on the
+ * residual augmented by a camera prior; cost(x) includes the prior's term).  With a prior, U, S and J include its rows:
+ * cov_cam = sigma2 (J_aug^T J_aug)^-1 restricted to the cameras.  S is rejected as rank deficient
  * when a pivot of its Cholesky factor has L_kk^2 <= 1e-12 U_kk; *min_pivot_ratio_out (may be NULL) receives the smallest
  * L_kk^2 / U_kk over the free camera slots.  The pivot test catches round-off pivots, it does not certify full rank: in
  * ill-conditioned geometry a single free direction (e.g. the scale left by one frozen perspective camera) can pass it, so
- * fix the gauge with at least two frozen cameras or with frozen points.  The handle stays usable for solves, also after an
- * error return. */
+ * fix the gauge with at least two frozen cameras, with frozen points, or with a camera prior (sba_problem_set_camera_prior):
+ * a prior of full rank on every free camera makes S positive definite by construction and gives the covariance of every
+ * camera, nothing frozen.  The handle stays usable for solves, also after an error return. */
 int sba_covariance(sba_problem *p, const double *x, int32_t loss, double f_scale, double sigma2,
                    double *cov_cam, double *cov_pts, double *sigma2_out, double *min_pivot_ratio_out);
 /* Device time (CUDA events) of the phases of the last sba_covariance call on this handle: reduced system (assembly, Schur

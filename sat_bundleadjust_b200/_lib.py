@@ -69,7 +69,7 @@ EXPORTED_SYMBOLS = [
     "sba_cholesky_solve_timed", "sba_outlier_elbow", "sba_outlier_mark",
     "sba_rpcfit_weighted_lsq", "sba_comm_export", "sba_comm_import", "sba_comm_try_reuse", "sba_solve_errors_device",
     "sba_init_pts3d", "sba_linear_triangulation", "sba_rpc_projection_batch", "sba_rpc_localization_batch",
-    "sba_covariance", "sba_covariance_phase_ms",
+    "sba_covariance", "sba_covariance_phase_ms", "sba_problem_set_camera_prior",
 ]
 
 _lib = None
@@ -104,6 +104,7 @@ def load():
     lib.sba_covariance.argtypes = [vp, c_double_p, ctypes.c_int32, ctypes.c_double, ctypes.c_double, c_double_p, c_double_p,
                                    c_double_p, c_double_p]
     lib.sba_covariance_phase_ms.argtypes = [vp, c_double_p]
+    lib.sba_problem_set_camera_prior.argtypes = [vp, c_double_p, c_double_p]
     lib.sba_solve.argtypes = [vp, c_double_p, ctypes.POINTER(SolveOpts), c_double_p, c_double_p, ctypes.POINTER(SolveInfo)]
     lib.sba_solve_device.argtypes = [vp, vp, ctypes.POINTER(SolveOpts), vp, vp, ctypes.POINTER(SolveInfo)]
     lib.sba_assemble_device.argtypes = [vp, vp, ctypes.c_int32, ctypes.c_double, c_float_p]

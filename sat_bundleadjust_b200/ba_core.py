@@ -93,13 +93,15 @@ def compute_mean_reprojection_error_per_track(err, pts_ind, cam_ind):
         return (s / cnt).astype(np.float32)
 
 
-def run_ba_optimization(p, ls_params=None, verbose=False, plots=True, return_info=False):
+def run_ba_optimization(p, ls_params=None, verbose=False, plots=True, return_info=False, cam_prior=None):
     """
     Solve the bundle adjustment problem on the GPU.
 
     Returns (vars_init, vars_ba, err_init, err_ba, iterations) exactly like the reference
     (`iterations` = number of residual evaluations, i.e. scipy's nfev).  `plots` is accepted for
     signature compatibility; figures are out of scope.  `return_info=True` appends the solver's info dict.
+    `cam_prior` (a ba_priors.CameraPrior) adds a Gaussian prior on the camera variables to the objective; the info's
+    cost_init / cost then include its term, err_init / err_ba stay the pixel errors of the observations.
     """
     cfg = init_optimization_config(ls_params)
     if verbose:
@@ -109,7 +111,7 @@ def run_ba_optimization(p, ls_params=None, verbose=False, plots=True, return_inf
     import time
     vars_init = initial_vars(p)
     t0 = time.perf_counter()
-    with DeviceProblem(p) as prob:
+    with DeviceProblem(p, cam_prior=cam_prior) as prob:
         t1 = time.perf_counter()
         try:
             vars_ba, err_init, err_ba, info = prob.solve_with_errors(

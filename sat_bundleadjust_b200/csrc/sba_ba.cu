@@ -13,6 +13,8 @@
 //     boundary (common.py:222-245); initial Delta = |x0 * scale_inv|             (trf.py:443)
 //   * termination: dF < ftol F with ratio > 0.25 | |dx| < xtol (xtol + |x|) | |g|_inf < gtol |
 //     nfev == max_nfev                                                           (common.py:705-717)
+// With a Gaussian prior on the camera variables (sba_problem_set_camera_prior, sba_prior.cuh) all of the above is that of the
+// augmented residual [r ; C_j (x_j - mu_j)], the loss applied to the observation rows only.
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
@@ -30,6 +32,7 @@
 #include "sba_kernels.cuh"
 #include "sba_pattern.cuh"
 #include "sba_pcg.cuh"
+#include "sba_prior.cuh"
 #include "sba_tr2d.h"
 
 namespace sba {
@@ -195,6 +198,27 @@ static int check_launch(sba_problem* p)
     return SBA_OK;
 }
 
+// the camera prior as the kernels see it: set only on rank 0, which adds it once before every exchange
+static CamPrior cam_prior(const sba_problem* p)
+{
+    CamPrior pr;
+    const bool on = p->has_prior && p->rank == 0;
+    pr.mean = on ? p->prior_mean : nullptr;
+    pr.info = on ? p->prior_info : nullptr;
+    return pr;
+}
+
+// generic engine: scal[s_cost] += the prior cost at x, scal[s11/s12/s22] += v1^T L v1, v1^T L v2, v2^T L v2 (slot < 0: skipped).
+// One small launch, only when a prior is set and only on rank 0.
+static int run_prior_scalars(sba_problem* p, const double* x, int s_cost, const double* v1, const double* v2, int s11, int s12,
+                             int s22)
+{
+    const CamPrior pr = cam_prior(p);
+    if (!pr.info) return SBA_OK;
+    k_prior_scalars<<<1, 256, 0, p->stream>>>(pr, p->M, p->nc, x, s_cost, v1, v2, s11, s12, s22, p->scal);
+    return check_launch(p);
+}
+
 // ---- per-phase / per-iteration device timing (CUDA events on the solver's stream) --------------------
 struct PhaseTimer {
     sba_problem* p;
@@ -285,6 +309,12 @@ static int run_assemble(sba_problem* p, const double* x, const double* camrec, i
         SBA_DISPATCH(p, L);
 #undef L
         SBA_TRY(check_launch(p));
+        const CamPrior pr = cam_prior(p);
+        if (pr.info) {       // camera prior: U_j += L_j, g_c,j += L_j (x_j - mu_j), on this rank's sums before the exchange
+            k_prior_cameras<<<grid_for((long long)p->M * p->nc, 256, NUM_SMS), 256, 0, p->stream2>>>(pr, x, p->M, p->nc,
+                                                                                                     p->camsys_local);
+            SBA_TRY(check_launch(p));
+        }
     }
     SBA_CUDA(cudaEventRecord(p->ev_join, p->stream2));
     {
@@ -584,6 +614,7 @@ static int trf_cost_x0(sba_problem* p, const sba_solve_opts* o)
     if (p->engine == 1) return pt_run_assemble(p, 1, 1, o->loss, o->f_scale);
     SBA_TRY(run_prepare(p, p->x, p->camrec));
     SBA_TRY(run_residual(p, p->x, p->camrec, o->loss, o->f_scale, nullptr, SC_COST_NEW, 0));
+    SBA_TRY(run_prior_scalars(p, p->x, SC_COST_NEW, nullptr, nullptr, -1, -1, -1));
     return allreduce_scal(p, SC_COST_NEW, 1);
 }
 
@@ -628,6 +659,7 @@ static int trf_step(sba_problem* p, const sba_solve_opts* o, PhaseTimer& tm, boo
         SBA_TRY(run_scale_dots(p, first ? 1 : 0));
         Slots sa; sa.s[0] = SC_A; sa.s[1] = SC_SCRATCH; sa.s[2] = SC_SCRATCH;
         SBA_TRY(run_jvp(p, loss, fs, 1, sa));
+        SBA_TRY(run_prior_scalars(p, p->x, SC_COST, p->t1, nullptr, SC_A, -1, -1));
         SBA_TRY(allreduce_scal(p, SC_COST, SC_GGN - SC_COST));
         tm.end();
     }
@@ -644,6 +676,7 @@ static int trf_step(sba_problem* p, const sba_solve_opts* o, PhaseTimer& tm, boo
     SBA_TRY(check_launch(p));
     Slots sb; sb.s[0] = SC_B11; sb.s[1] = SC_B12; sb.s[2] = SC_B22;
     SBA_TRY(run_jvp(p, loss, fs, 2, sb));
+    SBA_TRY(run_prior_scalars(p, nullptr, -1, p->t1, p->t2, SC_B11, SC_B12, SC_B22));
     SBA_TRY(allreduce_scal(p, SC_WW, 8));      // [ww wg t11 t12 t22 | b11 b12 b22] in one exchange
     tm.end();
     return SBA_OK;
@@ -666,6 +699,7 @@ static int trf_trial(sba_problem* p, const sba_solve_opts* o, double radius)
                                                                     p->model);
     SBA_TRY(check_launch(p));
     SBA_TRY(run_residual(p, p->x_new, p->camrec_new, o->loss, o->f_scale, nullptr, SC_COST_NEW, 0));
+    SBA_TRY(run_prior_scalars(p, p->x_new, SC_COST_NEW, nullptr, nullptr, -1, -1, -1));
     return allreduce_scal(p, SC_COST_NEW, 1);
 }
 
@@ -1165,6 +1199,87 @@ extern "C" int sba_problem_set_allreduce(sba_problem* p, sba_allreduce_fn fn, vo
     return SBA_OK;
 }
 
+// eigenvalues of the symmetric n x n matrix A (row-major, destroyed) by cyclic Jacobi sweeps; n <= 11 here
+static void sym_eigenvalues(double* A, int n, double* ev)
+{
+    for (int sweep = 0; sweep < 100; ++sweep) {
+        double off = 0.0, tot = 0.0;
+        for (int r = 0; r < n; ++r)
+            for (int c = 0; c < n; ++c) { tot += A[r * n + c] * A[r * n + c]; if (r != c) off += A[r * n + c] * A[r * n + c]; }
+        if (off <= 1e-30 * tot || off == 0.0) break;
+        for (int a = 0; a < n; ++a)
+            for (int b = a + 1; b < n; ++b) {
+                const double apq = A[a * n + b];
+                if (apq == 0.0) continue;
+                const double theta = (A[b * n + b] - A[a * n + a]) / (2.0 * apq);
+                const double t = (theta >= 0.0 ? 1.0 : -1.0) / (std::fabs(theta) + std::sqrt(theta * theta + 1.0));
+                const double cs = 1.0 / std::sqrt(t * t + 1.0), sn = t * cs;
+                for (int k = 0; k < n; ++k) {          // columns a, b
+                    const double ka = A[k * n + a], kb = A[k * n + b];
+                    A[k * n + a] = cs * ka - sn * kb;
+                    A[k * n + b] = sn * ka + cs * kb;
+                }
+                for (int k = 0; k < n; ++k) {          // rows a, b
+                    const double ak = A[a * n + k], bk = A[b * n + k];
+                    A[a * n + k] = cs * ak - sn * bk;
+                    A[b * n + k] = sn * ak + cs * bk;
+                }
+            }
+    }
+    for (int k = 0; k < n; ++k) ev[k] = A[k * n + k];
+}
+
+// Gaussian prior on the camera variables (sba_prior.cuh has the definitions).  Validated and symmetrised on the host, kept in
+// the problem's arena; NULL, NULL clears it.
+extern "C" int sba_problem_set_camera_prior(sba_problem* p, const double* mean, const double* info)
+{
+    if (!p) { set_error("null argument"); return SBA_E_INVALID; }
+    if (!mean && !info) { p->has_prior = false; p->prior_rank_sum = 0; return SBA_OK; }
+    if (!mean || !info) { set_error("sba_problem_set_camera_prior: give both the mean and the information, or neither"); return SBA_E_INVALID; }
+    if (p->n_common) { set_error("sba_problem_set_camera_prior: not available with shared calibration (n_common > 0)"); return SBA_E_INVALID; }
+    const int M = p->M, nc = p->nc;
+    const size_t ns = (size_t)M * nc;
+    std::vector<double> mu(mean, mean + ns), L(info, info + ns * nc);
+    for (double v : mu) if (!std::isfinite(v)) { set_error("sba_problem_set_camera_prior: non-finite mean"); return SBA_E_INVALID; }
+    for (double v : L) if (!std::isfinite(v)) { set_error("sba_problem_set_camera_prior: non-finite information"); return SBA_E_INVALID; }
+    long long rank_sum = 0;
+    std::vector<double> A((size_t)nc * nc), ev(nc);
+    for (int j = 0; j < M; ++j) {
+        double* Lj = L.data() + (size_t)j * nc * nc;
+        double amax = 0.0;
+        for (int k = 0; k < nc * nc; ++k) amax = std::max(amax, std::fabs(Lj[k]));
+        for (int r = 0; r < nc; ++r)
+            for (int c = r + 1; c < nc; ++c) {
+                if (std::fabs(Lj[r * nc + c] - Lj[c * nc + r]) > 1e-12 * amax) {
+                    set_error("sba_problem_set_camera_prior: information block of camera " + std::to_string(j) + " is not symmetric");
+                    return SBA_E_INVALID;
+                }
+                Lj[r * nc + c] = Lj[c * nc + r] = 0.5 * (Lj[r * nc + c] + Lj[c * nc + r]);
+            }
+        std::copy(Lj, Lj + nc * nc, A.begin());
+        sym_eigenvalues(A.data(), nc, ev.data());
+        const double emax = *std::max_element(ev.begin(), ev.end()), emin = *std::min_element(ev.begin(), ev.end());
+        if (emin < -1e-12 * std::max(emax, 0.0)) {
+            set_error("sba_problem_set_camera_prior: information block of camera " + std::to_string(j) +
+                      " is not positive semi-definite (eigenvalue " + std::to_string(emin) + ")");
+            return SBA_E_INVALID;
+        }
+        if (j < p->n_cam_fix) { std::fill(Lj, Lj + nc * nc, 0.0); continue; }      // frozen cameras: the prior is ignored
+        for (double e : ev) rank_sum += e > 1e-12 * emax;
+    }
+    SBA_CUDA(cudaSetDevice(p->device));
+    if (!p->prior_mean) {
+        SBA_TRY(dev_alloc(p, &p->prior_mean, ns));
+        SBA_TRY(dev_alloc(p, &p->prior_info, ns * nc));
+    }
+    SBA_CUDA(cudaMemcpyAsync(p->prior_mean, mu.data(), ns * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+    SBA_CUDA(cudaMemcpyAsync(p->prior_info, L.data(), ns * nc * sizeof(double), cudaMemcpyHostToDevice, p->stream));
+    SBA_CUDA(cudaStreamSynchronize(p->stream));       // the host vectors go out of scope
+    p->has_prior = true;
+    p->prior_rank_sum = rank_sum;
+    return SBA_OK;
+}
+
 extern "C" int64_t sba_problem_num_vars(const sba_problem* p) { return p ? p->n : -1; }
 extern "C" int sba_problem_engine(const sba_problem* p) { return p ? p->engine : -1; }
 extern "C" int sba_problem_solver(const sba_problem* p) { return p ? (p->use_pcg ? 1 : 0) : -1; }
@@ -1320,7 +1435,8 @@ extern "C" int sba_normal_blocks(sba_problem* p, const double* x, int32_t loss, 
 // evaluation): S = U + reg D_c^2 - W (V + reg D_p^2)^-1 W^T and rhs = -(g_c - W (V + reg D_p^2)^-1 g_p), COMMON_K folded.
 // Exposed for the parity tests of the Schur complement; host buffers, S is (M n_params)^2 column-major.
 // Device part: x (host) is uploaded (then `uploaded`, if given, is recorded); afterwards p->x / p->camrec hold x, p->camsys its
-// U blocks, p->S the system, and the cost at x is in scal[SC_COST_NEW] (pattern engine) or scal[SC_COST] (generic engine).
+// U blocks, p->S the system, and the cost at x is in scal[SC_COST_NEW] (pattern engine) or scal[SC_COST] (generic engine, observation
+// rows only: there the camera prior's cost is added by the iteration, not here).
 static int form_reduced_system(sba_problem* p, const double* x, int32_t loss, double f_scale, double reg,
                                cudaEvent_t uploaded = nullptr)
 {
@@ -1405,9 +1521,9 @@ extern "C" int sba_covariance(sba_problem* p, const double* x, int32_t loss, dou
     if (p->n_common) { set_error("sba_covariance: not available with shared calibration (n_common > 0)"); return SBA_E_INVALID; }
     const int M = p->M, nc = p->nc, ns = M * nc;
     const long long n_free = (long long)(M - p->n_cam_fix) * nc + 3LL * (p->N - p->n_pts_fix);
-    const long long dof = 2 * (long long)p->K - n_free;
+    const long long dof = 2 * (long long)p->K + p->prior_rank_sum - n_free;      // prior rows: the ranks of the free cameras' L_j
     if (!(sigma2 > 0.0) && dof <= 0) {
-        set_error("sba_covariance: " + std::to_string(dof) + " degrees of freedom (2 K - free variables): sigma^2 cannot be estimated");
+        set_error("sba_covariance: " + std::to_string(dof) + " degrees of freedom (2 K + prior ranks - free variables): sigma^2 cannot be estimated");
         return SBA_E_INVALID;
     }
     SBA_CUDA(cudaSetDevice(p->device));
@@ -1427,11 +1543,12 @@ extern "C" int sba_covariance(sba_problem* p, const double* x, int32_t loss, dou
     // left with the same buffer roles as before the call
     struct Unswap { sba_problem* p; ~Unswap() { if (p->engine == 1) pt_accept(p); } } unswap{p};
     // sigma2 estimated: the cost at x by the residual kernel of sba_residuals, in float64 like the Jacobian rows (rpc_float32 is
-    // for fun parity only).  sigma2 given: the assembly's own cost serves the finiteness check.
+    // for fun parity only), plus the camera prior's.  sigma2 given: the assembly's own cost serves the finiteness check.
     int cost_slot = p->engine == 1 ? SC_COST_NEW : SC_COST;
     if (!(sigma2 > 0.0)) {
         cost_slot = SC_SCRATCH;
         SBA_TRY(run_residual(p, p->x, p->camrec, loss, f_scale, nullptr, SC_SCRATCH, 0));
+        SBA_TRY(run_prior_scalars(p, p->x, SC_SCRATCH, nullptr, nullptr, -1, -1, -1));
     }
     SBA_CUDA(cudaEventRecord(p->cov_ev[1], s));
     // factor (frozen slots: identity rows of S) and pivot test

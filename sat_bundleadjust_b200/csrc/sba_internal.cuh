@@ -178,6 +178,11 @@ struct sba_problem {
     double *pt_records = nullptr;                                   // Schur records, one per (unit, pass)
     double *r_int = nullptr, *e_int = nullptr;                      // (2K), (K) residuals / errors in internal order
 
+    // ---- Gaussian prior on the camera variables (sba_problem_set_camera_prior, sba_prior.cuh), allocated on first use ----
+    bool has_prior = false;
+    double *prior_mean = nullptr, *prior_info = nullptr;           // (M nc), (M, nc, nc) symmetrised; frozen cameras' blocks 0
+    long long prior_rank_sum = 0;                                   // sum over the free cameras of rank(L_j): degrees of freedom it adds
+
     // ---- posterior covariance (sba_covariance), allocated by its first call ----
     double *cov_cam = nullptr, *cov_pts = nullptr;                  // (ns x ns) s2 S^-1, (N, 6) point blocks in the caller's order
     double *cov_diag = nullptr;                                     // pivot test: min ratio, rejected slot, its ratio; bad points

@@ -20,6 +20,7 @@
 #include "sba_comm.cuh"
 #include "sba_kernels.cuh"
 #include "sba_pattern.h"
+#include "sba_prior.cuh"
 
 namespace sba {
 
@@ -361,6 +362,8 @@ k_pt_assemble(PatView A, const double* __restrict__ x, const double* __restrict_
 // Sum of the per-CTA partials of k_pt_assemble -> camsys = [U (M, NC, NC) | g_c (M NC) | cost].  One CTA; one warp per
 // value, lanes stride over the CTAs, fixed shuffle tree.  fold != 0 (single GPU): also derive the camera scaling.
 //   dsq_c_new = first ? (diag U == 0 ? 1 : diag U) : max(dsq_c_cur, diag U)      (x_scale='jac', scipy common.py:598-610, squared)
+// A camera prior (sba_prior.cuh; pr.info != null on rank 0 only) is added to each value as it is written, before the exchange:
+// L_j to U_j, L_j (x_j - mu_j) to g_c,j and the prior cost to the cost slot, at the trial point x_cam that K1 wrote.
 __device__ __forceinline__ void cam_scale_dev(const double* __restrict__ camsys, const double* __restrict__ dsq_c_cur,
                                               int first, int M, int NC, double* __restrict__ dsq_c_new,
                                               double* __restrict__ idsq_c_new, double* __restrict__ g_new, double* scal)
@@ -381,7 +384,8 @@ template <int NC>
 __global__ void __launch_bounds__(256)
 k_pt_reduce_assemble(const double* __restrict__ partials, int n_cta, int M, double* __restrict__ camsys, int fold,
                      const double* __restrict__ dsq_c_cur, int first, double* __restrict__ dsq_c_new,
-                     double* __restrict__ idsq_c_new, double* __restrict__ g_new, double* scal, unsigned* counter, CommFused comm)
+                     double* __restrict__ idsq_c_new, double* __restrict__ g_new, double* scal, unsigned* counter, CommFused comm,
+                     CamPrior pr, const double* __restrict__ x_cam)
 {
     constexpr int NU = NC * (NC + 1) / 2, NV = NU + NC;
     const int lane = threadIdx.x & 31;
@@ -392,6 +396,7 @@ k_pt_reduce_assemble(const double* __restrict__ partials, int n_cta, int M, doub
         for (int b = lane; b < n_cta; b += 32) s += partials[(size_t)v * n_cta + b];
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+        if (pr.info && v == M * NV) s += prior_cost_warp(pr, M, NC, x_cam);
         if (lane == 0) {
             if (v == M * NV) {
                 camsys[(size_t)M * NC * NC + (size_t)M * NC] = s;
@@ -401,9 +406,11 @@ k_pt_reduce_assemble(const double* __restrict__ partials, int n_cta, int M, doub
                     int r = 0;
                     while ((r + 1) * (r + 2) / 2 <= q) ++r;
                     const int c = q - r * (r + 1) / 2;
+                    if (pr.info) s += pr.info[(size_t)j * NC * NC + r * NC + c];
                     camsys[(size_t)j * NC * NC + r * NC + c] = s;
                     camsys[(size_t)j * NC * NC + c * NC + r] = s;
                 } else {
+                    if (pr.info) s += prior_grad_row(pr, j, q - NU, NC, x_cam);
                     camsys[(size_t)M * NC * NC + (size_t)j * NC + (q - NU)] = s;
                 }
             }
@@ -480,7 +487,8 @@ __global__ void __launch_bounds__(PT_THREADS_LIGHT, 1)
 k_pt_jvp1(PatView A, const double* __restrict__ x, const double* __restrict__ camrec, const double* __restrict__ V,
           const double* __restrict__ g, const double* __restrict__ dsq_c, const double* __restrict__ idsq_c,
           double* __restrict__ dsq, double* __restrict__ idsq, const double2* __restrict__ osc, int first, int ns,
-          int count_cameras, int rank, double* partials, unsigned* counter, double* scal, int fold_ctl, double delta_arg, CommFused comm)
+          int count_cameras, int rank, double* partials, unsigned* counter, double* scal, int fold_ctl, double delta_arg, CommFused comm,
+          CamPrior pr)
 {
     extern __shared__ double smem[];
     double* s_cam = smem;
@@ -501,6 +509,7 @@ k_pt_jvp1(PatView A, const double* __restrict__ x, const double* __restrict__ ca
             acc[2] += xv * xv;
             gmax = fmax(gmax, fabs(gv));
         }
+        if (pr.info) acc[3] += prior_forms_rows(pr, ns, NC, s_t1c, s_t1c).x;      // camera prior: + t1^T L t1
     }
     const int u0 = A.warp_unit0[blockIdx.x * nw + warp], u1 = A.debug_skip ? u0 : A.warp_unit0[blockIdx.x * nw + warp + 1];
     const long long cyc0 = clock64();
@@ -1162,7 +1171,7 @@ k_pt_backsub(PatView A, const double* __restrict__ x, const double* __restrict__
              const double* __restrict__ g, const double* __restrict__ dsq, const double* __restrict__ idsq,
              const double* __restrict__ dsq_c, const double* __restrict__ idsq_c, const double2* __restrict__ osc,
              double* __restrict__ delta, int ns, int count_cameras, double* partials, unsigned* counter, double* scal, int fold_ctl,
-             CommFused comm)
+             CommFused comm, CamPrior pr)
 {
     extern __shared__ double smem[];
     double* s_cam = smem;
@@ -1181,6 +1190,11 @@ k_pt_backsub(PatView A, const double* __restrict__ x, const double* __restrict__
         for (int e = threadIdx.x; e < ns; e += blockDim.x) {
             const double d = s_dc[e], t = s_t1c[e];
             acc[0] += g[e] * d; acc[1] += dsq_c[e] * d * d; acc[4] += t * t; acc[5] += t * d; acc[6] += d * d;
+        }
+        if (pr.info) {                                  // camera prior: + t1^T L delta, + delta^T L delta
+            const double2 q = prior_forms_rows(pr, ns, NC, s_t1c, s_dc);
+            acc[2] += q.x;
+            acc[3] += q.y;
         }
     }
     double* stg = s_stage + warp * 3 * 32;

@@ -54,11 +54,13 @@ class _CudaView:
         self.__cuda_array_interface__ = {"shape": (count,), "typestr": "<f8", "data": (ptr, False), "version": 2}
 
 
-def run_ba_optimization_distributed(p, ls_params=None, group=None):
+def run_ba_optimization_distributed(p, ls_params=None, group=None, cam_prior=None):
     """
     Multi-GPU counterpart of ba_core.run_ba_optimization, to be called by every rank of an initialised
     torch.distributed NCCL process group (one process per GPU).  Every rank passes the same `p`.
     Returns (vars_init, vars_ba, err_init, err_ba, nfev, info) with the global vectors on every rank.
+    `cam_prior` (a ba_priors.CameraPrior, the same on every rank) adds a Gaussian prior on the camera variables; rank 0's
+    kernels add its terms once, before each exchange.
 
     Each rank uploads only its own shard, the per-iteration exchanges run over NVLink peer memory, and the results
     (x, err_init, err of every shard) are all-gathered on the device and brought back with one copy into pinned memory.
@@ -132,6 +134,8 @@ def run_ba_optimization_distributed(p, ls_params=None, group=None):
         prob = DeviceProblem(p, stream=stream, rank=rank, world_size=world, track_range=ranges[rank],
                              engine="pattern" if lo_l[0] else "generic", solver="dense" if lo_l[1] else "pcg")
     with prob:
+        if cam_prior is not None:                      # after the re-create above: every rank, on the handle that solves
+            prob.set_camera_prior(cam_prior)
         t_create = time.perf_counter()
         prob.set_allreduce(hook)                       # NCCL fall-back for exchanges that do not fit the peer buffer
         if os.environ.get("SBA_COMM", "peer") == "peer":

@@ -75,8 +75,10 @@ def from_device_layout(x, n_common, n_params, n_cam):
 class DeviceProblem:
     """RAII wrapper of sba_problem_create / sba_problem_destroy."""
 
-    def __init__(self, p, stream=0, rank=0, world_size=1, rpc_float32=True, track_range=None, engine=None, solver=None):
-        """engine: None (automatic) | "pattern" | "generic";  solver: None (automatic) | "dense" | "pcg"."""
+    def __init__(self, p, stream=0, rank=0, world_size=1, rpc_float32=True, track_range=None, engine=None, solver=None,
+                 cam_prior=None):
+        """engine: None (automatic) | "pattern" | "generic";  solver: None (automatic) | "dense" | "pcg";
+        cam_prior: None or a ba_priors.CameraPrior (see set_camera_prior)."""
         check_supported(p)
         self.lib = _lib.load()
         self.cam_model = p.cam_model
@@ -119,6 +121,27 @@ class DeviceProblem:
         # length of the caller's vector (the reference's params_opt layout); the device keeps n_params slots per camera
         self.n_vars = self.n_vars_device - (self.n_cam - 1) * self.n_common
         self._cb = None
+        self.cam_prior = None
+        if cam_prior is not None:
+            self.set_camera_prior(cam_prior)
+
+    def set_camera_prior(self, prior):
+        """
+        Gaussian prior on the camera variables (sat_bundleadjust_b200.ba_priors.CameraPrior) for the following solves,
+        normal_blocks, reduced_system and covariance of this handle; None clears it.  residuals() stays the observation rows.
+        """
+        if prior is None:
+            check(self.lib.sba_problem_set_camera_prior(self.handle, None, None))
+            self.cam_prior = None
+            return
+        if self.n_common:
+            raise NotImplementedError("camera priors are not available with COMMON_K (shared calibration)")
+        if prior.mean.shape != (self.n_cam, self.n_params):
+            raise ValueError("CameraPrior: mean is %s, the problem has (n_cam, n_params) = (%d, %d)"
+                             % (prior.mean.shape, self.n_cam, self.n_params))
+        mean, info = f64(prior.mean), f64(prior.information)
+        check(self.lib.sba_problem_set_camera_prior(self.handle, dptr(mean), dptr(info)))
+        self.cam_prior = prior
 
     def close(self):
         if getattr(self, "handle", None):
@@ -201,8 +224,9 @@ class DeviceProblem:
         """
         self._no_common("covariance")
         n_free = (self.n_cam - self._n_cam_fix) * self.n_params + 3 * (self.n_pts - self._fixed_pts.size // 3)
-        if not (sigma2 is not None and sigma2 > 0) and 2 * self.n_obs - n_free <= 0:
-            raise ValueError("no degrees of freedom left (2 K - n_free = %d): sigma^2 cannot be estimated" % (2 * self.n_obs - n_free))
+        dof = 2 * self.n_obs + (self.cam_prior.free_rank(self._n_cam_fix) if self.cam_prior is not None else 0) - n_free
+        if not (sigma2 is not None and sigma2 > 0) and dof <= 0:
+            raise ValueError("no degrees of freedom left (2 K + prior ranks - n_free = %d): sigma^2 cannot be estimated" % dof)
         x = self._vars(x)
         ns = self.n_cam * self.n_params
         cov_cam = np.empty((ns, ns), order="F")
