@@ -16,32 +16,9 @@ from oracle import ba_oracle, rpc_oracle
 from sat_bundleadjust_b200 import _lib, synth
 from sat_bundleadjust_b200.ba_covariance import compute_covariance, degrees_of_freedom
 from sat_bundleadjust_b200.solver import DeviceProblem, initial_vars
+from util import cond_tol, normalised_err as _normalised_err, scaled_cond, scaled_inv
 
 NORM_TOL = 1e-7
-EPS = np.finfo(np.float64).eps
-
-
-def scaled_cond(S, u_diag):
-    """2-norm condition number of S in the basis scaled by the un-reduced diagonal U_kk (numpy, oracle side)."""
-    d = np.sqrt(u_diag)
-    return np.linalg.cond(S / np.outer(d, d)) if S.size else 1.0
-
-
-def cond_tol(base, kappa, n):
-    """
-    The bound for a float64 S^-1: the issue's fixed bound, or the forward-error bound n eps kappa of a Cholesky-based inverse
-    (n free camera slots, kappa = scaled_cond of S from the oracle), whichever is larger.  S = U - W V^-1 W^T is formed by
-    cancellation against U, so its scaled entries carry ~eps of round-off whatever the method; satellite geometry is
-    ill-conditioned by nature (a narrow-field camera's rotation and translation nearly coincide), kappa ~ 1e9 .. 1e11 here,
-    which makes the fixed 1e-7 (1e-9 at the metric size) unreachable there.
-    """
-    return max(base, n * EPS * kappa)
-
-
-def scaled_inv(A):
-    """inverse in the Jacobi-scaled basis (accurate for badly scaled SPD matrices)"""
-    d = np.sqrt(np.diag(A))
-    return np.linalg.inv(A / np.outer(d, d)) / np.outer(d, d)
 
 
 PIVOT_THRESHOLD = 1e-12
@@ -57,16 +34,6 @@ def _robust_rows(J, f, loss, f_scale):
     rho = construct_loss_function(f.size, loss, f_scale)(f.copy())
     Js, _ = scale_for_robust_loss_function(J.copy(), f.copy(), rho)
     return Js
-
-
-def _normalised_err(A, B):
-    d = np.sqrt(np.abs(np.diag(B)))
-    den = np.outer(d, d)
-    mask = den > 0
-    err = np.zeros_like(A)
-    err[mask] = np.abs(A - B)[mask] / den[mask]
-    assert not np.abs(A - B)[~mask].any(), "entries where the oracle's variances are 0 must be exactly 0"
-    return err.max() if err.size else 0.0
 
 
 def oracle_residuals(x, p):

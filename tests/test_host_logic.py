@@ -449,24 +449,7 @@ def test_host_index_rejects_bad_input(built):
     assert _host_index([0, 1], [0, 7], 3, 3)[0] == 1                # track out of range
 
 
-def _pattern_layout(cam_ind, pts_ind, M, N, n_pts_fix=0, n_cta=148, warps=16):
-    import ctypes
-    lib = ctypes.CDLL(os.path.join(os.path.dirname(os.path.abspath(__file__)), "host_harness", "libmodel_harness.so"))
-    ip = ctypes.POINTER(ctypes.c_int)
-    cam = np.ascontiguousarray(cam_ind, dtype=np.int32)
-    tp = np.ascontiguousarray(np.searchsorted(pts_ind, np.arange(N + 1), side="left"), dtype=np.int32)
-    K = cam.size
-    sizes = (ctypes.c_int * 8)()
-    null = ctypes.cast(None, ip)
-    args = [cam.ctypes.data_as(ip), tp.ctypes.data_as(ip), ctypes.c_longlong(K), M, N, n_pts_fix, n_cta, warps, sizes]
-    lib.hh_pattern_layout(*args, *([null] * 5))
-    if not sizes[0]:
-        return None
-    out = {"trk_new2old": np.zeros(N, np.int32), "obs_new2old": np.zeros(K, np.int32), "track_ptr": np.zeros(N + 1, np.int32),
-           "units": np.zeros((sizes[1], 8), np.int32), "warp_unit0": np.zeros(n_cta * warps + 1, np.int32)}
-    lib.hh_pattern_layout(*args, *[out[k].ctypes.data_as(ip) for k in ("trk_new2old", "obs_new2old", "track_ptr", "units", "warp_unit0")])
-    out["n_frozen"], out["n_tiles"], out["n_runs"], out["fill"] = sizes[3], sizes[4], sizes[5], sizes[6] / 1000.0
-    return out
+_pattern_layout = util.pattern_layout
 
 
 @pytest.mark.parametrize("M,N,p_vis,fix", [(10, 100000, 0.5, 0), (10, 5000, 0.5, 37), (22, 3000, 0.3, 0), (3, 50, 0.5, 5), (6, 2000, 0.9, 0)])
